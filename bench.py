@@ -1,11 +1,18 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the vanilla-NeRF ray-march path (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--mode fp32|bf16] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--mode fp32|bf16] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one optimisation step of `train_nerf.py --vanilla` (train/trainer.py:702-729): stratified
 coarse sampling, coarse pass, sample_pdf + merge, fine pass, loss, backward, Adam -- over one batch of
 1024 synthetic Blender-shaped rays per GPU.  Prints ONE JSON line (rank 0).
+
+--dump-outputs DIR writes what the last of the K timed steps produced (rank 0) as float32 .npy files, so that two
+builds run with the same arguments -- hence the same seeded batches, weights and draws -- can be compared array by array.
+Repeated runs of one build are not bitwise identical: the backward sums with fp32 atomics, and Adam's early steps
+(~lr * sign(g)) amplify that where a gradient is near zero.  Two bf16 runs of the defaults on one B200 (1000 W limit)
+differed by about 6e-5 relative in the loss and up to about 6e-3 in single weights of magnitude <= 0.31 (about 1e-3 at
+the 99th percentile): profiles/r3_dump_repeatability.json.
 """
 import argparse
 import json
@@ -82,7 +89,7 @@ def llff_ndc_rays(rng, n):
 
 
 def dropin_rays_per_s(mode, dev, batches, steps=20, fuse=True):
-    """rays/s of the loop body train/trainer.py:702-725 executed by the REFERENCE'S code (baseline/_ref) on this package's
+    """rays/s of the loop body train/trainer.py:702-725 executed by the REFERENCE'S code (oracle/_ref) on this package's
     kernels: install(mode) rebinds its by-name imports, then its unbound Trainer._train_step, autograd backward and
     torch.optim.Adam run unmodified (amp off: the arithmetic mode is the kernels')."""
     import torch
@@ -181,15 +188,15 @@ def host_threads():
 
 def cpu_reference_step_fn(rays_per_step):
     """One full optimisation step (fwd+bwd+Adam) of the path on the host cores, on `rays_per_step` rays of the bench
-    workload.  Preferred: the reference's OWN code from baseline/_ref (unbound Trainer._train_step + backward + torch Adam,
-    fp32, amp off as the reference runs on a CPU device) -> kind "reference".  Only when baseline/_ref is absent: the numpy
+    workload.  Preferred: the reference's OWN code from oracle/_ref (unbound Trainer._train_step + backward + torch Adam,
+    fp32, amp off as the reference runs on a CPU device) -> kind "reference".  Only when oracle/_ref is absent: the numpy
     oracle port -> kind "port".  Returns (step callable, kind, threads actually used, description)."""
     threads = host_threads()
     rng = np.random.default_rng(0)
     from baseline import ref_runner
     if ref_runner.available():
         step, info = ref_runner.make_cpu_step(lambda i: blender_rays(rng, rays_per_step, i), nc=NC, nf=NF, threads=threads)
-        return step, "reference", info["threads"], (f"reference Trainer._train_step + backward + torch.optim.Adam (baseline/_ref, unmodified), "
+        return step, "reference", info["threads"], (f"reference Trainer._train_step + backward + torch.optim.Adam (oracle/_ref, unmodified), "
                                                     f"torch {info['torch']} CPU fp32, torch threads={info['threads']}")
     from threadpoolctl import threadpool_limits
     from oracle import nerf_oracle as O
@@ -209,7 +216,15 @@ def cpu_reference_step_fn(rays_per_step):
         st["Pf"], st["m"][2], st["m"][3] = O.adam_step(st["Pf"], O.flatten_params(out["grads_f"]), st["m"][2], st["m"][3], st["t"])
         st["pc"], st["pf"] = O.unflatten_params(st["Pc"]), O.unflatten_params(st["Pf"])
         return float(out["loss"])
-    return step, "port", threads, f"numpy fp32 oracle port (baseline/_ref absent), BLAS threads={threads}"
+    return step, "port", threads, f"numpy fp32 oracle port (oracle/_ref absent), BLAS threads={threads}"
+
+
+def dump_outputs(out_dir, tr):
+    """The step's scalars [loss, psnr, mse_c, mse_f] and the parameters it updated in place (2 x 595,844 fp32, 4.8 MB)."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"scalars": tr.scalars, "params_coarse": tr.nerf_c.flat_params(), "params_fine": tr.nerf_f.flat_params()}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 WORKLOAD = ("vanilla NeRF Blender-shape training 800x800 white bkgd precrop, 1024 rays/step/GPU, 64 coarse + 128 fine, "
@@ -244,7 +259,9 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of each training loop (headline, end to end, repeats, LLFF-NDC, drop-in); the field "
+                         "roofline times a fixed 10 launch sets and the CPU baseline a fixed 4 steps")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--mode", default=os.environ.get("NSB_BENCH_MODE", "bf16"), choices=["fp32", "bf16"])
@@ -253,7 +270,12 @@ def main():
     ap.add_argument("--no-cfg4", action="store_true")
     ap.add_argument("--no-dropin", action="store_true")
     ap.add_argument("--graph", type=int, default=1, help="capture the step in a CUDA graph (N=1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -316,6 +338,8 @@ def main():
     else:
         launches = _lib.launch_count() - l0 + (K if world > 1 and tr.peer is None else 0)      # + one NCCL all-reduce kernel per step
     loss_dev = float(tr.scalars[0])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, tr)
     # ---- end to end: pinned host batch -> H2D -> step -> D2H loss, every step ---------------------------
     # one pinned host buffer per batch, [o | d | norm | viewdir | rgb] field-major, so a step is ONE H2D copy
     keys = ("rays_o_marching", "rays_d_marching_unit", "rays_d_marching_norm", "rays_d_world_unit", "rgb")
@@ -445,16 +469,15 @@ def main():
         for i in range(3):
             step4(pool4[i % 4])
         barrier()
-        K4 = 10
         e0.record()
-        for i in range(K4):
+        for i in range(K):
             step4(pool4[i % 4])
         e1.record()
         barrier()
-        ms4 = max_over_ranks(e0.elapsed_time(e1)) / K4
+        ms4 = max_over_ranks(e0.elapsed_time(e1)) / K
         extra["cfg4"] = {"workload": "LLFF fern-shape NDC (504x378, f=407.6, z in [0,1]) training, 8192 rays/step/GPU, 64+128 (BASELINE configs[3])",
                          "rays_per_step_per_gpu": B4, "n_gpus": world, "ms_per_step": ms4, "train_rays_per_s": world * B4 / (ms4 * 1e-3),
-                         "steps": K4, "loss_after": float(tr4.scalars[0]),
+                         "steps": K, "loss_after": float(tr4.scalars[0]),
                          "mlp_tflops_per_gpu": B4 * POINTS_PER_RAY * FLOP_TRAIN_PER_POINT / (ms4 * 1e-3) / 1e12}
         tr4.check_peers()
         del tr4, pool4
@@ -463,9 +486,9 @@ def main():
     # ---- the drop-in seam: the REFERENCE'S OWN Trainer._train_step + backward + torch Adam after install(mode) (N=1) -------
     if rank == 0 and world == 1 and not args.no_dropin:
         try:      # install()'s default (Trainer._train_step = the fused step) and the reference's own _train_step body
-            extra["dropin"] = dropin_rays_per_s(args.mode, dev, devb)
-            extra["dropin_reference_body"] = dropin_rays_per_s(args.mode, dev, devb, fuse=False)
-        except Exception as exc:                      # baseline/_ref absent, ...: report, do not fail the bench
+            extra["dropin"] = dropin_rays_per_s(args.mode, dev, devb, steps=K)
+            extra["dropin_reference_body"] = dropin_rays_per_s(args.mode, dev, devb, steps=K, fuse=False)
+        except Exception as exc:                      # oracle/_ref absent, ...: report, do not fail the bench
             extra["dropin"] = {"unavailable": repr(exc)[:200]}
 
     # ---- CPU baseline (rank 0, N=1 only): the oracle port on the host cores, bounded sample ---------------
@@ -489,7 +512,7 @@ def main():
                 render()
                 t0 = time.perf_counter(); render(); dt = time.perf_counter() - t0
                 extra["render_cpu_baseline"] = {"rays_per_s": tile / dt, "frames_per_s_extrapolated": tile / dt / (H * W), "cores": info["threads"],
-                                                "kind": "reference", "sample": f"render_image_chunked (baseline/_ref, unmodified) on a {tile}-ray tile, "
+                                                "kind": "reference", "sample": f"render_image_chunked (oracle/_ref, unmodified) on a {tile}-ray tile, "
                                                 f"64 + 128 samples, fp32 CPU, second of two calls"}
             except Exception as exc:
                 extra["render_cpu_baseline"] = {"unavailable": repr(exc)[:200]}

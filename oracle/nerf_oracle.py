@@ -10,7 +10,7 @@ Where the arithmetic lives: the reference delegates every op to PyTorch/ATen
 (``requirements.txt:2`` lists ``torch`` unpinned; 2.11.0 in this image).  Each
 function below restates the ATen op sequence of the cited reference lines in
 numpy float32.  Parity pin: ``tests/make_golden.py`` imports the reference from
-``/root/reference`` in the build container, runs it on seeded inputs and
+its checkout (``NSB_REFERENCE_SRC``, else BASELINE.json's ``reference_path``), runs it on seeded inputs and
 commits the input/output vectors under ``tests/golden/``;
 ``tests/test_oracle_golden.py`` checks this file against them (bit-exact for
 ``sample_pdf`` bin indices and the stratified/merge samplers, <=2e-6 for the

@@ -1,5 +1,5 @@
 """Generate tests/golden/*.npz by running the UNMODIFIED reference (evan-wes/nerf-sandbox)
-on seeded inputs.  Runs only in the build container (needs /root/reference); the
+on seeded inputs.  Needs a checkout of the reference (NSB_REFERENCE_SRC, else BASELINE.json's reference_path); the
 fixtures it writes are committed and are what pins oracle/nerf_oracle.py.
 
     python tests/make_golden.py            # rewrites tests/golden/
@@ -22,7 +22,11 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 sys.path.insert(0, ROOT)
-sys.path.insert(0, "/root/reference")
+from baseline import ref_runner  # noqa: E402
+REF_CHECKOUT = ref_runner.reference_checkout()
+if not os.path.isdir(os.path.join(REF_CHECKOUT, "nerf_sandbox")):
+    sys.exit(f"no reference checkout at {REF_CHECKOUT}: set NSB_REFERENCE_SRC to a checkout of evan-wes/nerf-sandbox")
+sys.path.insert(0, REF_CHECKOUT)
 
 # imageio is not installed and is imported at module scope by render_utils.py:20
 _shim = types.ModuleType("imageio"); _shim.v2 = types.ModuleType("imageio.v2")

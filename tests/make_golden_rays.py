@@ -1,9 +1,14 @@
-"""tests/golden/rays.npz from the unmodified reference get_camera_rays (utils/ray_utils.py).  Build container only."""
+"""tests/golden/rays.npz from the unmodified reference get_camera_rays (utils/ray_utils.py).  Needs a reference checkout (see make_golden.py)."""
 import os, sys
 import numpy as np
 import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, os.path.dirname(HERE))
+from baseline import ref_runner  # noqa: E402
+REF_CHECKOUT = ref_runner.reference_checkout()
+if not os.path.isdir(os.path.join(REF_CHECKOUT, "nerf_sandbox")):
+    sys.exit(f"no reference checkout at {REF_CHECKOUT}: set NSB_REFERENCE_SRC to a checkout of evan-wes/nerf-sandbox")
+sys.path.insert(0, REF_CHECKOUT)
 from nerf_sandbox.source.utils.ray_utils import get_camera_rays  # noqa: E402
 
 rng = np.random.default_rng(77)

@@ -1,4 +1,4 @@
-"""The drop-in seam, driven by the REFERENCE'S OWN code (baseline/_ref = the unmodified reference package, vendored by
+"""The drop-in seam, driven by the REFERENCE'S OWN code (oracle/_ref = the unmodified reference package, vendored by
 __graft_entry__.build()): after ``install()`` the reference's ``Trainer._train_step`` and its whole
 ``train_nerf.py --vanilla`` entry point run on the libnsb kernels.
 
@@ -35,7 +35,7 @@ def N(t):
 def ref():
     from baseline import ref_runner
     if not ref_runner.available():
-        pytest.skip("baseline/_ref missing (run __graft_entry__.build() in the build container)")
+        pytest.skip("oracle/_ref holds no reference (vendored by __graft_entry__.build() from NSB_REFERENCE_SRC, else BASELINE.json's reference_path)")
     TR, RU = ref_runner.import_reference()
     yield ref_runner, TR, RU
     from nerf_sandbox_b200.install import uninstall

@@ -45,16 +45,16 @@ def test_scene_ground_truth_is_a_valid_image():
 
 
 def test_reference_arm_runs_the_vendored_reference():
-    """bench.py --impl reference / cpu_baseline: the reference's own Trainer._train_step + backward + Adam (baseline/_ref)."""
+    """bench.py --impl reference / cpu_baseline: the reference's own Trainer._train_step + backward + Adam (oracle/_ref)."""
     from baseline import ref_runner
     if not ref_runner.available():
-        pytest.skip("baseline/_ref missing (vendored by __graft_entry__.build() where /root/reference exists)")
+        pytest.skip("oracle/_ref holds no reference (vendored by __graft_entry__.build() from NSB_REFERENCE_SRC, else BASELINE.json's reference_path)")
     rng = np.random.default_rng(0)
     step, info = ref_runner.make_cpu_step(lambda i: O.synthetic_rays(rng, 32), nc=16, nf=16, threads=2)
     l0 = step(); l1 = step()
     assert np.isfinite([l0, l1]).all() and info["threads"] == 2
     # unmodified: the vendored files are byte-identical to the reference checkout when that is present
-    src = "/root/reference/nerf_sandbox/source/train/trainer.py"
+    src = os.path.join(ref_runner.reference_checkout(), "nerf_sandbox", "source", "train", "trainer.py")
     if os.path.isfile(src):
         assert open(src, "rb").read() == open(os.path.join(ref_runner.REF_DIR, "nerf_sandbox/source/train/trainer.py"), "rb").read()
 

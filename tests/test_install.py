@@ -1,14 +1,14 @@
 """The drop-in seam: install() rebinds the reference's by-name imports (only where the reference is present)."""
-import os
 import sys
 
 import pytest
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "baseline", "_ref")          # the unmodified reference package, vendored by __graft_entry__.build()
+from baseline import ref_runner
+
+REF = ref_runner.REF_DIR          # the unmodified reference package, vendored by __graft_entry__.build()
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "nerf_sandbox")), reason="baseline/_ref not vendored")
+@pytest.mark.skipif(not ref_runner.available(), reason="oracle/_ref holds no reference")
 def test_install_rebinds_reference_names():
     sys.path.insert(0, REF)
     try:
