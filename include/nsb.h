@@ -109,6 +109,13 @@ int nsb_composite_raw_fwd(const float* raw, const float* noise, float noise_std,
 int nsb_composite_raw_bwd(const float* raw, const float* noise, float noise_std, const float* z,
                           const float* ray_norm, const float* g_comp, float* d_raw, int64_t B, int N,
                           uint32_t flags, uint64_t seed, uint64_t offset, void* stream);
+/* The same with the gradients of every output of volume_render_rays (render_utils.py:141-167): g_comp[B,3], g_weights[B,N],
+ * g_acc[B], g_depth[B], each [opt] (a missing one counts as zero), at least one given -- a depth or opacity loss, or a loss on
+ * the weights, reaches the field through d_raw.  nsb_composite_raw_bwd is this call with g_comp only.  No gradient w.r.t. z or
+ * ray_norm. */
+int nsb_composite_raw_bwd_ex(const float* raw, const float* noise, float noise_std, const float* z, const float* ray_norm,
+                             const float* g_comp, const float* g_weights, const float* g_acc, const float* g_depth, float* d_raw,
+                             int64_t B, int N, uint32_t flags, uint64_t seed, uint64_t offset, void* stream);
 
 /* nsb_composite_raw_bwd with the step's loss gradient formed in place (train/trainer.py:999-1004 + :717): instead of g_comp it
  * takes target[B,3] and loss_scale = 2 * grad_scale / (3 * B_total), and uses dL/dcomp = (guard(comp) - guard(target)) *
@@ -131,6 +138,17 @@ int nsb_mse_loss(const float* comp_c, const float* comp_f, const float* target, 
 /* PositionalEncoder.forward, models/encoders.py:73-106.  x[Q,D] -> out[Q, D*(include_input + 2L)],
  * order [x | sin(2^k x_d) k-major | cos(...)]. */
 int nsb_encode(const float* x, float* out, int64_t Q, int D, int L, int include_input, void* stream);
+/* Its autograd (encoders.py:101-104 through torch's sin/cos backward): g_out[Q, D*(include_input + 2L)] -> g_x[Q,D] =
+ * [include_input] g + sum_k 2^k (cos(2^k x) g_sin_k - sin(2^k x) g_cos_k). */
+int nsb_encode_bwd(const float* x, const float* g_out, float* g_x, int64_t Q, int D, int L, int include_input, void* stream);
+/* Backward of the points + encodings step of nerf_forward_pass (render_utils.py:211-223, gamma(x) with L = 10, gamma(d) with
+ * L = 4, both with the input): d_enc_pos[B*N,63], d_enc_dir[B*N,27] -> d_rays_o[B,3] = sum over samples of d pts,
+ * d_rays_d[B,3] = sum of d pts * (z * norm), and the view-direction term through F.normalize's backward (eps 1e-12) into
+ * d_viewdirs[B,3], or into d_rays_d when viewdirs is NULL.  Outputs [opt], at least one.  Inputs as nsb_field_fwd_rays.
+ * Sums run in a fixed order (no atomics): bitwise repeatable.  z and ray_norm get no gradient. */
+int nsb_encode_bwd_rays(const float* d_enc_pos, const float* d_enc_dir, const float* rays_o, const float* rays_d, const float* z,
+                        const float* ray_norm, const float* viewdirs, float* d_rays_o, float* d_rays_d, float* d_viewdirs,
+                        int64_t B, int N, void* stream);
 
 /* Packed weights of one NeRF: fp32 padded rows for the FFMA path, and images in tcgen05 operand layout for the tensor
  * paths -- bf16 (training forward), transposed bf16 (dgrad), fp16 (inference forward) and the fp16 low halves of the
@@ -164,9 +182,15 @@ int nsb_field_fwd_rays(const float* rays_o, const float* rays_d, const float* z,
                        int64_t B, int N, int mode, int stash, void* stream);
 
 /* Parameter gradients of the pass whose activations are stashed in ws: grads[NSB_N_PARAMS] (flat,
- * state_dict order) += dL/dparams given d_raw[Q,4].  Inputs carry no gradient (SURVEY 8 a12). */
+ * state_dict order) += dL/dparams given d_raw[Q,4].  (nsb_field_bwd_ex with no input gradients.) */
 int nsb_field_bwd(const float* d_raw, const void* packed, float* grads, void* ws, size_t ws_bytes,
                   int64_t Q, int mode, void* stream);
+/* NeRF.forward's autograd w.r.t. its parameters AND its inputs (mlps.py:221-278): grads [opt] as above, d_enc_pos[Q,63] [opt] and
+ * d_enc_dir[Q,27] [opt] are overwritten with dL/d gamma(x) = dY_0 W_0[:, 0:63] + dY_4 W_4[:, 256:319] (layer 4's input is
+ * [h, gamma(x)], mlps.py:224-227) and dL/d gamma(d) = dY_9 W_cfc[:, 256:283] (dY_l = gradient of layer l's pre-activation).
+ * At least one output.  grads == NULL is a frozen field: no weight-gradient kernel runs at all. */
+int nsb_field_bwd_ex(const float* d_raw, const void* packed, float* grads, float* d_enc_pos, float* d_enc_dir, void* ws,
+                     size_t ws_bytes, int64_t Q, int mode, void* stream);
 
 /* torch.optim.Adam step (train/trainer.py:383-386, :722) on flat buffers; grads are multiplied by
  * grad_scale first (1/world_size after a sum-allreduce). t is the 1-based step count.

@@ -36,9 +36,12 @@ SIGNATURES = {
     "nsb_composite_bwd": (_i32, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _i32, _u32, _f32, _p]),
     "nsb_composite_raw_fwd": (_i32, [_p, _p, _f32, _p, _p, _p, _p, _p, _p, _i64, _i32, _u32, _u64, _u64, _p]),
     "nsb_composite_raw_bwd": (_i32, [_p, _p, _f32, _p, _p, _p, _p, _i64, _i32, _u32, _u64, _u64, _p]),
+    "nsb_composite_raw_bwd_ex": (_i32, [_p, _p, _f32, _p, _p, _p, _p, _p, _p, _p, _i64, _i32, _u32, _u64, _u64, _p]),
     "nsb_composite_raw_bwd_mse": (_i32, [_p, _p, _f32, _p, _p, _p, _f32, _p, _i64, _i32, _u32, _u64, _u64, _p]),
     "nsb_mse_loss": (_i32, [_p, _p, _p, _p, _p, _p, _i64, _f32, _p]),
     "nsb_encode": (_i32, [_p, _p, _i64, _i32, _i32, _i32, _p]),
+    "nsb_encode_bwd": (_i32, [_p, _p, _p, _i64, _i32, _i32, _i32, _p]),
+    "nsb_encode_bwd_rays": (_i32, [_p] * 10 + [_i64, _i32, _p]),
     "nsb_packed_weights_bytes": (_sz, []),
     "nsb_pack_weights": (_i32, [_p, _p, _i32, _p]),
     "nsb_pack_weights_batch": (_i32, [_p, _p, _i32, _i32, _p]),
@@ -46,6 +49,7 @@ SIGNATURES = {
     "nsb_field_fwd_enc": (_i32, [_p, _p, _p, _p, _p, _sz, _i64, _i32, _i32, _p]),
     "nsb_field_fwd_rays": (_i32, [_p, _p, _p, _p, _p, _p, _p, _p, _sz, _i64, _i32, _i32, _i32, _p]),
     "nsb_field_bwd": (_i32, [_p, _p, _p, _p, _sz, _i64, _i32, _p]),
+    "nsb_field_bwd_ex": (_i32, [_p, _p, _p, _p, _p, _p, _sz, _i64, _i32, _p]),
     "nsb_adam_step": (_i32, [_p, _p, _p, _p, _i64, _f32, _f32, _f32, _f32, _i64, _f32, _p, _p]),
     "nsb_grad_clip": (_i32, [_p, _i64, _f32, _f32, _p, _p]),
     "nsb_adam_allreduce_step": (_i32, [_p, _p, _p, _i32, _p, _p, _p, _p, _p, _p, _i32, _i32, _u32, _i64, _f32, _f32, _f32, _f32, _i64, _f32, _p, _p]),

@@ -65,7 +65,7 @@ __device__ __forceinline__ float finalize_color(float c) {   // :165 nan_to_num(
 // posinf=1, neginf=0).clamp(0,1); loss_scale = 2 * grad_scale / (3 B).  (The composite's own clamp mask is applied by the caller.)
 __device__ __forceinline__ float comp_grad(const float* __restrict__ g_comp, const float* __restrict__ target, float loss_scale, float craw,
                                            int64_t i) {
-    if (!target) return __ldg(g_comp + i);
+    if (!target) return g_comp ? __ldg(g_comp + i) : 0.0f;             // a missing g_comp counts as zero
     float t = __ldg(target + i);
     if (isnan(t)) t = 0.0f;
     t = fminf(fmaxf(t, 0.0f), 1.0f);
@@ -901,16 +901,24 @@ extern "C" int nsb_composite_raw_bwd_mse(const float* raw, const float* noise, f
                             seed, offset, stream, 0, target, loss_scale);
 }
 
+extern "C" int nsb_composite_raw_bwd_ex(const float* raw, const float* noise, float noise_std, const float* z, const float* ray_norm,
+                                        const float* g_comp, const float* g_weights, const float* g_acc, const float* g_depth, float* d_raw,
+                                        int64_t B, int N, uint32_t flags, uint64_t seed, uint64_t offset, void* stream) {
+    if (B == 0) return NSB_OK;
+    if (!raw || !z || !d_raw || N < 1 || B < 0 || (!g_comp && !g_weights && !g_acc && !g_depth)) return NSB_E_BADARG;
+    if (N <= kRunMaxN)
+        return launch_bwd_run<true>(raw, nullptr, noise, noise_std, z, ray_norm, g_comp, g_weights, g_acc, g_depth, d_raw, nullptr, B, N, flags,
+                                    1e-10f, seed, offset, stream);
+    return launch_bwd<true>(raw, nullptr, noise, noise_std, z, ray_norm, g_comp, g_weights, g_acc, g_depth, d_raw,
+                            nullptr, B, N, flags, 1e-10f, seed, offset, stream);
+}
+
 extern "C" int nsb_composite_raw_bwd(const float* raw, const float* noise, float noise_std, const float* z,
                                      const float* ray_norm, const float* g_comp, float* d_raw, int64_t B, int N,
                                      uint32_t flags, uint64_t seed, uint64_t offset, void* stream) {
-    if (B == 0) return NSB_OK;
-    if (!raw || !z || !g_comp || !d_raw || N < 1 || B < 0) return NSB_E_BADARG;
-    if (N <= kRunMaxN)
-        return launch_bwd_run<true>(raw, nullptr, noise, noise_std, z, ray_norm, g_comp, nullptr, nullptr, nullptr, d_raw, nullptr, B, N, flags,
-                                    1e-10f, seed, offset, stream);
-    return launch_bwd<true>(raw, nullptr, noise, noise_std, z, ray_norm, g_comp, nullptr, nullptr, nullptr, d_raw,
-                            nullptr, B, N, flags, 1e-10f, seed, offset, stream);
+    if (B != 0 && !g_comp) return NSB_E_BADARG;
+    return nsb_composite_raw_bwd_ex(raw, noise, noise_std, z, ray_norm, g_comp, nullptr, nullptr, nullptr, d_raw, B, N, flags, seed, offset,
+                                    stream);
 }
 
 extern "C" int nsb_mse_loss(const float* comp_c, const float* comp_f, const float* target, float* g_c, float* g_f,

@@ -38,7 +38,8 @@ int pack_fp32(const float* params, void* packed, cudaStream_t st);
 int fp32_prepare_rays(const float*, const float*, const float*, const float*, const float*, void*, int64_t, int, int, cudaStream_t);
 int fp32_prepare_enc(const float*, const float*, void*, int64_t, int, cudaStream_t);
 int fp32_mlp_fwd(const void* packed, float* raw, void* ws, int64_t Q, int stash, cudaStream_t st);
-int fp32_mlp_bwd(const float* d_raw, const void* packed, float* grads, void* ws, int64_t Q, cudaStream_t st);
+int fp32_mlp_bwd(const float* d_raw, const void* packed, float* grads, float* d_enc_pos, float* d_enc_dir, void* ws, int64_t Q,
+                 cudaStream_t st);
 // field_tc.cu
 size_t tc_workspace_bytes(int64_t Q, int stash);
 size_t tc_stash_tile_bytes();
@@ -49,7 +50,8 @@ int tc_field_fwd_rays(const float*, const float*, const float*, const float*, co
                       float* raw, void* ws, int64_t B, int N, int stash, cudaStream_t st);
 int tc_field_fwd_enc(const float* enc_pos, const float* enc_dir, const void* packed, float* raw, void* ws, int64_t Q,
                      int stash, cudaStream_t st);
-int tc_field_bwd(const float* d_raw, const void* packed, float* grads, void* ws, int64_t Q, cudaStream_t st);
+int tc_field_bwd(const float* d_raw, const void* packed, float* grads, float* d_enc_pos, float* d_enc_dir, void* ws, int64_t Q,
+                 cudaStream_t st);
 
 int tc_field_fwd_rays_split(const float*, const float*, const float*, const float*, const float*, const void* packed, float* raw,
                             int64_t B, int N, cudaStream_t st);
@@ -144,15 +146,21 @@ extern "C" int nsb_field_fwd_rays(const float* rays_o, const float* rays_d, cons
     return fp32_mlp_fwd(packed, raw, ws, Q, stash, as_stream(stream));
 }
 
-extern "C" int nsb_field_bwd(const float* d_raw, const void* packed, float* grads, void* ws, size_t ws_bytes, int64_t Q,
-                             int mode, void* stream) {
+extern "C" int nsb_field_bwd_ex(const float* d_raw, const void* packed, float* grads, float* d_enc_pos, float* d_enc_dir, void* ws,
+                                size_t ws_bytes, int64_t Q, int mode, void* stream) {
     if (Q == 0) return NSB_OK;
-    if (!d_raw || !packed || !grads || !ws || Q < 0) return NSB_E_BADARG;
+    if (!d_raw || !packed || !ws || Q < 0 || (!grads && !d_enc_pos && !d_enc_dir)) return NSB_E_BADARG;
     if (ws_bytes < field_ws(Q, mode, 1)) return NSB_E_WORKSPACE;
     if (mode == NSB_MODE_BF16)
-        return tc_field_bwd(d_raw, reinterpret_cast<const char*>(packed) + packed_layout().bf16_off, grads, ws, Q,
+        return tc_field_bwd(d_raw, reinterpret_cast<const char*>(packed) + packed_layout().bf16_off, grads, d_enc_pos, d_enc_dir, ws, Q,
                             as_stream(stream));
-    return fp32_mlp_bwd(d_raw, packed, grads, ws, Q, as_stream(stream));
+    return fp32_mlp_bwd(d_raw, packed, grads, d_enc_pos, d_enc_dir, ws, Q, as_stream(stream));
+}
+
+extern "C" int nsb_field_bwd(const float* d_raw, const void* packed, float* grads, void* ws, size_t ws_bytes, int64_t Q,
+                             int mode, void* stream) {
+    if (Q != 0 && !grads) return NSB_E_BADARG;
+    return nsb_field_bwd_ex(d_raw, packed, grads, nullptr, nullptr, ws, ws_bytes, Q, mode, stream);
 }
 
 // test hook (not part of include/nsb.h): tensor-core forward + fp32 dump of one layer's activations [Q,256]

@@ -78,6 +78,99 @@ __global__ void encode_kernel(const float* __restrict__ x, float* __restrict__ o
     }
 }
 
+// PositionalEncoder backward: g_x[q,d] = [include] g[q,d] + sum_k 2^k (cos(2^k x) g_sin[k,d] - sin(2^k x) g_cos[k,d]), in the output
+// order of encode_kernel; thread per (q, d).  sincosf is the accurate one, as in the forward: arguments reach 2^9 |x|.
+__global__ void encode_bwd_kernel(const float* __restrict__ x, const float* __restrict__ g, float* __restrict__ gx, int64_t Q, int D, int L,
+                                  int include_input) {
+    const int od = D * (include_input ? 1 : 0) + 2 * L * D, o0 = include_input ? D : 0;
+    for (int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; idx < Q * D; idx += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t q = idx / D;
+        const int d = (int)(idx % D);
+        const float* gr = g + q * od;
+        const float xv = x[idx];
+        float acc = include_input ? gr[d] : 0.f;
+        for (int k = 0; k < L; ++k) {
+            const float f = exp2f((float)k);
+            float sn, cs;
+            sincosf(xv * f, &sn, &cs);
+            acc += f * (cs * gr[o0 + k * D + d] - sn * gr[o0 + L * D + k * D + d]);
+        }
+        gx[idx] = acc;
+    }
+}
+
+// Backward of the points + encodings step of nerf_forward_pass (render_utils.py:211-223) for gamma(x) (L = 10) and gamma(d)
+// (L = 4), include_input, D = 3.  One warp per ray: lane i takes samples i, i + 32, ...; the sums over samples run in that fixed
+// order and then through a fixed butterfly, so the input gradients are bitwise repeatable (no atomics).
+//   pts = o + d * (z * norm)   ->  d_o = sum dx,  d_d = sum dx * (z * norm)
+//   v = normalize(viewdirs or d, eps 1e-12)  ->  F.normalize backward of sum dv, into d_viewdirs (or d_d when viewdirs is null)
+__global__ void __launch_bounds__(256)
+encode_bwd_rays_kernel(const float* __restrict__ d_enc_pos, const float* __restrict__ d_enc_dir, const float* __restrict__ rays_o,
+                       const float* __restrict__ rays_d, const float* __restrict__ z, const float* __restrict__ ray_norm,
+                       const float* __restrict__ viewdirs, float* __restrict__ d_rays_o, float* __restrict__ d_rays_d,
+                       float* __restrict__ d_viewdirs, int64_t B, int N) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warp = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
+    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t b = warp; b < B; b += nwarps) {
+        const float o[3] = {rays_o[b * 3 + 0], rays_o[b * 3 + 1], rays_o[b * 3 + 2]};
+        const float dd[3] = {rays_d[b * 3 + 0], rays_d[b * 3 + 1], rays_d[b * 3 + 2]};
+        const float* vsrc = viewdirs ? viewdirs : rays_d;
+        const float vr[3] = {vsrc[b * 3 + 0], vsrc[b * 3 + 1], vsrc[b * 3 + 2]};
+        const float nv = sqrtf(vr[0] * vr[0] + vr[1] * vr[1] + vr[2] * vr[2]);
+        const float nrm = fmaxf(nv, 1e-12f);
+        const float v[3] = {vr[0] / nrm, vr[1] / nrm, vr[2] / nrm};
+        float sx[3] = {0.f, 0.f, 0.f}, sxz[3] = {0.f, 0.f, 0.f}, sv[3] = {0.f, 0.f, 0.f};
+        for (int i = lane; i < N; i += 32) {
+            const int64_t q = b * N + i;
+            const float zm = ray_norm ? __fmul_rn(z[q], ray_norm[b]) : z[q];
+            const float* gp = d_enc_pos + q * kPosDim;
+            const float* gd = d_enc_dir + q * kDirDim;
+#pragma unroll
+            for (int d = 0; d < 3; ++d) {
+                const float p = __fadd_rn(o[d], __fmul_rn(dd[d], zm));
+                float ax = gp[d];
+#pragma unroll
+                for (int k = 0; k < 10; ++k) {
+                    const float f = exp2f((float)k);
+                    float sn, cs;
+                    sincosf(p * f, &sn, &cs);
+                    ax += f * (cs * gp[3 + 3 * k + d] - sn * gp[33 + 3 * k + d]);
+                }
+                float av = gd[d];
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    const float f = exp2f((float)k);
+                    float sn, cs;
+                    sincosf(v[d] * f, &sn, &cs);
+                    av += f * (cs * gd[3 + 3 * k + d] - sn * gd[15 + 3 * k + d]);
+                }
+                sx[d] += ax; sxz[d] += ax * zm; sv[d] += av;
+            }
+        }
+#pragma unroll
+        for (int d = 0; d < 3; ++d) { sx[d] = warp_sum(sx[d]); sxz[d] = warp_sum(sxz[d]); sv[d] = warp_sum(sv[d]); }
+        if (lane == 0) {
+            // F.normalize: v = x / max(|x|, eps) -> dx = (g - v (v . g)) / |x| when |x| > eps, else g / eps
+            float gvx[3];
+            if (nv > 1e-12f) {
+                const float vg = v[0] * sv[0] + v[1] * sv[1] + v[2] * sv[2];
+#pragma unroll
+                for (int d = 0; d < 3; ++d) gvx[d] = (sv[d] - v[d] * vg) / nv;
+            } else {
+#pragma unroll
+                for (int d = 0; d < 3; ++d) gvx[d] = sv[d] / 1e-12f;
+            }
+#pragma unroll
+            for (int d = 0; d < 3; ++d) {
+                if (d_rays_o) d_rays_o[b * 3 + d] = sx[d];
+                if (d_rays_d) d_rays_d[b * 3 + d] = sxz[d] + (viewdirs ? 0.f : gvx[d]);
+                if (d_viewdirs && viewdirs) d_viewdirs[b * 3 + d] = gvx[d];
+            }
+        }
+    }
+}
+
 // points + both encodings into the padded activation buffers; 16 threads per point
 __global__ void prepare_from_rays_kernel(const float* __restrict__ rays_o, const float* __restrict__ rays_d,
                                          const float* __restrict__ z, const float* __restrict__ ray_norm,
@@ -252,6 +345,10 @@ __global__ void __launch_bounds__(256) sgemm_kernel(GemmArgs g) {
                 v[0] += bb.x; v[1] += bb.y; v[2] += bb.z; v[3] += bb.w;
                 if (g.relu) { v[0] = fmaxf(v[0], 0.f); v[1] = fmaxf(v[1], 0.f); v[2] = fmaxf(v[2], 0.f); v[3] = fmaxf(v[3], 0.f); }
                 *reinterpret_cast<float4*>(g.C + m * g.ldc + n) = make_float4(v[0], v[1], v[2], v[3]);
+            } else if (EPI == EPI_DGRAD && g.n_valid > 0) {
+#pragma unroll
+                for (int j = 0; j < 4; ++j)
+                    if (n + j < g.n_valid) g.C[m * g.ldc + n + j] = v[j] + (g.addend ? g.addend[m * g.ldadd + n + j] : 0.f);
             } else if (EPI == EPI_DGRAD) {
                 if (g.addend) {
                     const float4 ad = *reinterpret_cast<const float4*>(g.addend + m * g.ldadd + n);
@@ -347,6 +444,7 @@ head_bwd_kernel(const float* __restrict__ d_raw, const float* __restrict__ C, co
         as1.x += d.w * h1.x; as1.y += d.w * h1.y; as1.z += d.w * h1.z; as1.w += d.w * h1.w;
         if (lane == 0) { b0 += d.x; b1 += d.y; b2 += d.z; bsig += d.w; }
     }
+    if (gWo == nullptr) return;          // frozen field: input gradients only
     // block-level reduction in shared memory, then one atomic per element per block
     __shared__ float red[3 * 128 + 256 + 4];
     for (int i = threadIdx.x; i < 3 * 128 + 256 + 4; i += blockDim.x) red[i] = 0.f;
@@ -406,6 +504,10 @@ PackedLayout packed_layout() {
         L.split_fwd[l] = off; off += align_up(split_image_bytes(d.N, d.Kpad), 256);
         if (l > 0) { L.split_dgrad[l] = off; off += align_up(split_image_bytes(kHidden, d.N), 256); }
     }
+    for (int i = 0; i < 3; ++i) {                              // W_0[:, 0:63]^T, W_4[:, 256:319]^T (64 rows), W_cfc[:, 256:283]^T (32)
+        L.split_dinput[i] = off;
+        off += align_up(split_image_bytes(i < 2 ? 64 : 32, i < 2 ? kHidden : kColorHidden), 256);
+    }
     L.split_bytes = off - L.split_off;
     L.total = off;
     return L;
@@ -460,6 +562,19 @@ static int gemm_dgrad(const float* dY, int64_t ldy, const float* W, const uint8_
     dim3 grid((unsigned)cdiv(Q, BM), (unsigned)cdiv(n_in, BN), 1);
     sgemm_kernel<false, true, EPI_DGRAD><<<grid, 256, 0, st>>>(g);
     NSB_LAUNCH_CHECK("sgemm_dgrad");
+    return NSB_OK;
+}
+// Input gradient: dE[Q, n_valid] (row stride lde, any) = dY[Q, n_out] . W[n_out, ldw] (n_in columns from W, n_in a multiple of 16
+// covering n_valid; the padding columns of W are zero) (+ addend, same layout as dE)
+static int gemm_dinput(const float* dY, int64_t ldy, const float* W, const uint8_t* w_img, int ldw, float* dE, int64_t lde, int64_t Q,
+                       int n_out, int n_in, int n_valid, const float* addend, cudaStream_t st) {
+    GemmArgs g{};
+    g.A = dY; g.lda = ldy; g.B = W; g.ldb = ldw; g.C = dE; g.ldc = lde; g.Mdim = Q; g.Ndim = n_in; g.Kdim = n_out;
+    g.addend = addend; g.ldadd = lde; g.n_valid = n_valid; g.b_img = w_img;
+    if (gemm_on_tc()) return split_gemm(g, EPI_DGRAD, st);
+    dim3 grid((unsigned)cdiv(Q, BM), (unsigned)cdiv(n_in, BN), 1);
+    sgemm_kernel<false, true, EPI_DGRAD><<<grid, 256, 0, st>>>(g);
+    NSB_LAUNCH_CHECK("sgemm_dinput");
     return NSB_OK;
 }
 // gW[n_out, K] += dY[Q, n_out]^T . X[Q, Kpad] ; gb[n_out] += colsum(dY)
@@ -531,29 +646,43 @@ int fp32_mlp_fwd(const void* packed, float* raw, void* ws, int64_t Q, int stash,
     return NSB_OK;
 }
 
-// parameter grads (accumulated into flat `grads`) from the stashed activations
-int fp32_mlp_bwd(const float* d_raw, const void* packed, float* grads, void* ws, int64_t Q, cudaStream_t st) {
+// Parameter grads (accumulated into flat `grads`, or none when it is null: a frozen field) and the gradients w.r.t. the two
+// encodings (d_enc_pos [Q,63], d_enc_dir [Q,27], each optional) from the stashed activations:
+//   d gamma(d) = dY_9 . W_cfc[:, 256:283],   d gamma(x) = dY_0 . W_0 + dY_4 . W_4[:, 256:319]   (layer 4's input is [h | gamma(x)])
+int fp32_mlp_bwd(const float* d_raw, const void* packed, float* grads, float* d_enc_pos, float* d_enc_dir, void* ws, int64_t Q,
+                 cudaStream_t st) {
     const PackedLayout L = packed_layout();
     Fp32Ws w = carve_fp32(ws, Q, 1);
     const float* H8 = w.out[7];
     const LayerDesc dsg = layer_desc(9), dco = layer_desc(11), dfc = layer_desc(10), dft = layer_desc(8);
+    auto G = [&](int64_t off) { return grads ? grads + off : nullptr; };
     int hb_grid = num_sms() * 4;
     if ((int64_t)hb_grid * 8 > Q) hb_grid = (int)cdiv(Q, 8);
     head_bwd_kernel<<<hb_grid, 256, 0, st>>>(d_raw, w.C, H8, kHidden, PW(packed, L, 11), PW(packed, L, 9), w.dC, w.dA,
-                                             grads + dco.w_off, grads + dco.b_off, grads + dsg.w_off, grads + dsg.b_off, Q);
+                                             G(dco.w_off), G(dco.b_off), G(dsg.w_off), G(dsg.b_off), Q);
     NSB_LAUNCH_CHECK("head_bwd_kernel");
+    if (d_enc_dir)
+        NSB_TRY(gemm_dinput(w.dC, kColorHidden, PW(packed, L, 10) + kHidden, IMG(packed, L.split_dinput[2]), kColorPad, d_enc_dir, kDirDim, Q,
+                            kColorHidden, 32, kDirDim, nullptr, st));
+    if (!grads && !d_enc_pos) return NSB_OK;
     // color_fc
-    NSB_TRY(gemm_wgrad(w.dC, kColorHidden, w.XC, kColorPad, grads + dfc.w_off, grads + dfc.b_off, Q, 128, dfc.K, dfc.Kpad, st));
+    if (grads) NSB_TRY(gemm_wgrad(w.dC, kColorHidden, w.XC, kColorPad, grads + dfc.w_off, grads + dfc.b_off, Q, 128, dfc.K, dfc.Kpad, st));
     NSB_TRY(gemm_dgrad(w.dC, kColorHidden, PW(packed, L, 10), IMG(packed, L.split_dgrad[10]), kColorPad, w.dB, kHidden, Q, 128, 256, nullptr, 0, nullptr, 0, st));  // dFeat
     // feature (no activation); dH8 = (dFeat.Wf + dsigma*w_sigma) * (H8>0)
-    NSB_TRY(gemm_wgrad(w.dB, kHidden, H8, kHidden, grads + dft.w_off, grads + dft.b_off, Q, 256, 256, 256, st));
+    if (grads) NSB_TRY(gemm_wgrad(w.dB, kHidden, H8, kHidden, grads + dft.w_off, grads + dft.b_off, Q, 256, 256, 256, st));
     NSB_TRY(gemm_dgrad(w.dB, kHidden, PW(packed, L, 8), IMG(packed, L.split_dgrad[8]), 256, w.dA, kHidden, Q, 256, 256, H8, kHidden, w.dA, kHidden, st));
     float* dcur = w.dA; float* dnext = w.dB;
     for (int l = 7; l >= 0; --l) {
         const LayerDesc d = layer_desc(l);
         const float* Xin = l == 0 ? w.X0 : (l == 4 ? w.X4 : w.out[l - 1]);
         const int64_t ldx = l == 0 ? kPosPad : (l == 4 ? kSkipPad : w.out_ld[l - 1]);
-        NSB_TRY(gemm_wgrad(dcur, kHidden, Xin, ldx, grads + d.w_off, grads + d.b_off, Q, 256, d.K, d.Kpad, st));
+        if (grads) NSB_TRY(gemm_wgrad(dcur, kHidden, Xin, ldx, grads + d.w_off, grads + d.b_off, Q, 256, d.K, d.Kpad, st));
+        if (d_enc_pos && l == 4)        // the gamma(x) slab of the skip input, before the ping-pong overwrites dY_4
+            NSB_TRY(gemm_dinput(dcur, kHidden, PW(packed, L, 4) + kHidden, IMG(packed, L.split_dinput[1]), kSkipPad, d_enc_pos, kPosDim, Q,
+                                kHidden, kPosPad, kPosDim, nullptr, st));
+        if (d_enc_pos && l == 0)
+            NSB_TRY(gemm_dinput(dcur, kHidden, PW(packed, L, 0), IMG(packed, L.split_dinput[0]), kPosPad, d_enc_pos, kPosDim, Q, kHidden, kPosPad,
+                                kPosDim, d_enc_pos, st));
         if (l > 0) {
             // input of layer l is relu(out[l-1]) -> mask by out[l-1] > 0 (first 256 columns only at the skip layer)
             NSB_TRY(gemm_dgrad(dcur, kHidden, PW(packed, L, l), IMG(packed, L.split_dgrad[l]), d.Kpad, dnext, kHidden, Q, 256, 256, w.out[l - 1],
@@ -909,6 +1038,26 @@ extern "C" int nsb_encode(const float* x, float* out, int64_t Q, int D, int L, i
     const int od = D * (include_input ? 1 : 0) + 2 * L * D;
     encode_kernel<<<elem_grid(Q * od), 256, 0, as_stream(stream)>>>(x, out, Q, D, L, include_input);
     NSB_LAUNCH_CHECK("encode_kernel");
+    return NSB_OK;
+}
+
+extern "C" int nsb_encode_bwd(const float* x, const float* g_out, float* g_x, int64_t Q, int D, int L, int include_input, void* stream) {
+    if (Q == 0) return NSB_OK;
+    if (!x || !g_out || !g_x || Q < 0 || D < 1 || L < 0) return NSB_E_BADARG;
+    encode_bwd_kernel<<<elem_grid(Q * D), 256, 0, as_stream(stream)>>>(x, g_out, g_x, Q, D, L, include_input);
+    NSB_LAUNCH_CHECK("encode_bwd_kernel");
+    return NSB_OK;
+}
+
+extern "C" int nsb_encode_bwd_rays(const float* d_enc_pos, const float* d_enc_dir, const float* rays_o, const float* rays_d, const float* z,
+                                   const float* ray_norm, const float* viewdirs, float* d_rays_o, float* d_rays_d, float* d_viewdirs,
+                                   int64_t B, int N, void* stream) {
+    if (B == 0) return NSB_OK;
+    if (!d_enc_pos || !d_enc_dir || !rays_o || !rays_d || !z || B < 0 || N < 1) return NSB_E_BADARG;
+    if (!d_rays_o && !d_rays_d && !d_viewdirs) return NSB_E_BADARG;
+    encode_bwd_rays_kernel<<<elem_grid(B * 32), 256, 0, as_stream(stream)>>>(d_enc_pos, d_enc_dir, rays_o, rays_d, z, ray_norm, viewdirs,
+                                                                          d_rays_o, d_rays_d, d_viewdirs, B, N);
+    NSB_LAUNCH_CHECK("encode_bwd_rays_kernel");
     return NSB_OK;
 }
 

@@ -307,6 +307,16 @@ __global__ void __launch_bounds__(SG_THREADS, BN == 128 ? 2 : 1) split_gemm_kern
                     if (nn < g.n_valid) atomicAdd(g.C + m * g.ldc + nn, tile_s[r * LD + 32 * q + lane]);
                 }
             }
+        } else if (EPI == EPI_DGRAD && g.n_valid > 0) {
+            // input gradients: columns < n_valid of an output with any row stride, one warp per row, lane = column
+            for (int r = warp; r < SG_BM; r += SG_CONV / 32) {
+                const int64_t m = m0 + r;
+                if (m >= g.Mdim) break;
+                for (int c = lane; c < BN; c += 32) {
+                    const int64_t nn = n0 + c;
+                    if (nn < g.n_valid) g.C[m * g.ldc + nn] = tile_s[r * LD + c] + (g.addend ? g.addend[m * g.ldadd + nn] : 0.f);
+                }
+            }
         } else if (BN == 128 && n < g.Ndim) {
             float4 bb = make_float4(0.f, 0.f, 0.f, 0.f);
             if (EPI == EPI_FWD) bb = __ldg(reinterpret_cast<const float4*>(g.bias + n));
@@ -344,7 +354,7 @@ __global__ void __launch_bounds__(SG_THREADS, BN == 128 ? 2 : 1) split_gemm_kern
 // (a multiple of 16), element = W[n * ldw + k] (transpose = 0) or W[k * ldw + n] (transpose = 1), zero where k >= k_true
 // (n >= n_true).  Layout: [n / 128][k / 16][term][(k / 8) % 2][n % 128][k % 8] bf16.
 struct SplitPackJob { int64_t w_off; int ldw; int transpose; int n_true, k_true, n_tiles, k_chunks; size_t dst; };
-constexpr int kSplitJobs = 19;
+constexpr int kSplitJobs = 22;
 struct SplitPackArgs { SplitPackJob j[kSplitJobs]; };
 __global__ void __launch_bounds__(256) split_pack_kernel(const float* __restrict__ params, uint8_t* __restrict__ base, const __grid_constant__ SplitPackArgs a) {
     const SplitPackJob& jb = a.j[blockIdx.y];
@@ -409,7 +419,8 @@ static int split_terms() {
 size_t split_image_bytes(int n_rows, int k_len) { return (size_t)cdiv(n_rows, 128) * (size_t)(k_len / 16) * tc::SG_IMG_CHUNK; }
 
 // Every weight image of a net: forward B = W (n = out feature, k = in feature, zero beyond K), dgrad B = W^T restricted to
-// the first 256 in features (n = in feature, k = out feature).  One launch, 19 jobs; ~7 MB written per net.
+// the first 256 in features (n = in feature, k = out feature), and W^T of the three input slices.  One launch, 22 jobs; ~7 MB
+// written per net.
 int split_pack(const float* params, void* packed, cudaStream_t st) {
     const PackedLayout L = packed_layout();
     tc::SplitPackArgs a;
@@ -420,6 +431,11 @@ int split_pack(const float* params, void* packed, cudaStream_t st) {
         a.j[nj++] = tc::SplitPackJob{d.w_off, d.K, 0, d.N, d.K, (int)cdiv(d.N, 128), d.Kpad / 16, L.split_fwd[l]};
         if (l > 0) a.j[nj++] = tc::SplitPackJob{d.w_off, d.K, 1, kHidden, d.N, kHidden / 128, d.N / 16, L.split_dgrad[l]};
     }
+    // input slices (dgrad B = W^T rows n = in feature): gamma(x) columns of mlp.0 and mlp.4, gamma(d) columns of color_fc
+    const LayerDesc d0 = layer_desc(0), d4 = layer_desc(4), dc = layer_desc(10);
+    a.j[nj++] = tc::SplitPackJob{d0.w_off, d0.K, 1, kPosDim, d0.N, 1, d0.N / 16, L.split_dinput[0]};
+    a.j[nj++] = tc::SplitPackJob{d4.w_off + kHidden, d4.K, 1, kPosDim, d4.N, 1, d4.N / 16, L.split_dinput[1]};
+    a.j[nj++] = tc::SplitPackJob{dc.w_off + kHidden, dc.K, 1, kDirDim, dc.N, 1, dc.N / 16, L.split_dinput[2]};
     if (nj != tc::kSplitJobs) return NSB_E_BADARG;
     tc::split_pack_kernel<<<dim3(16, tc::kSplitJobs), 256, 0, st>>>(params, reinterpret_cast<uint8_t*>(packed), a);
     NSB_LAUNCH_CHECK("split_pack_kernel");
@@ -435,7 +451,8 @@ static bool wgrad_wide() {
 int split_gemm(const GemmArgs& g, int role, cudaStream_t st) {
     NSB_TRY(check_arch());
     // alignment contract of the loaders / epilogues (all layer buffers of field_fp32.cu satisfy it)
-    if ((g.lda & 3) || (g.ldb & 3) || (role != EPI_WGRAD && ((g.Kdim & 15) || (g.ldc & 3) || (g.Ndim & 15)))) return NSB_E_BADARG;
+    const bool any_ldc = role == EPI_DGRAD && g.n_valid > 0;        // input gradients: scalar epilogue, any row stride
+    if ((g.lda & 3) || (g.ldb & 3) || (role != EPI_WGRAD && ((g.Kdim & 15) || ((g.ldc & 3) && !any_ldc) || (g.Ndim & 15)))) return NSB_E_BADARG;
     const bool t3 = split_terms() == 3;
     const bool img = g.b_img != nullptr && role != EPI_WGRAD;
 #define NSB_SG(AT, BT, EPI, IMGF) (t3 ? tc::launch_split_gemm<AT, BT, EPI, 3, IMGF>(g, st) : tc::launch_split_gemm<AT, BT, EPI, 2, IMGF>(g, st))

@@ -76,7 +76,11 @@ constexpr uint32_t kF16ImgOfs = kTImgOfs + 65536 + 8 * 131072;
 static_assert(kF16ImgOfs % 256 == 0 && kWeightImageBytes % 256 == 0, "images are addressed as rows of 256 B");
 // low halves of the fp16 SPLIT  w = hi + lo  (hi = the fp16 image above, lo = fp16(w - hi)) for the fp32-accurate forward
 constexpr uint32_t kF16LoImgOfs = kF16ImgOfs + kWeightImageBytes;
-constexpr uint32_t kPackedTcBytes = kF16LoImgOfs + kWeightImageBytes;
+// B operands of the input-gradient products (field_dinput_kernel), bf16 K-major images [k/8][rows][8] with k = out feature:
+//   W_0[:, 0:63]^T (64 rows, K = 256) | W_4[:, 256:319]^T (64 rows, K = 256) | W_cfc[:, 256:283]^T (32 rows, K = 128); padding zero
+constexpr uint32_t kDinImgOfs = kF16LoImgOfs + kWeightImageBytes;
+constexpr uint32_t kDinPos0 = 0, kDinPos4 = 32768, kDinDir = 65536, kDinImgBytes = 73728;
+constexpr uint32_t kPackedTcBytes = kDinImgOfs + kDinImgBytes;
 
 __host__ __device__ inline int layer_nslabs(int l) { return l == 0 ? 2 : (l == 4 ? 10 : (l == 9 ? 9 : 8)); }
 __host__ __device__ inline int layer_N(int l) { return l == 9 ? 128 : 256; }
@@ -1535,6 +1539,178 @@ __global__ void __launch_bounds__(kWgThreads, 1) field_wgrad_kernel(const __grid
     }
 }
 
+// =======================================================================================================
+// Backward, part 3 (only when input gradients are asked for): gradients w.r.t. the two encodings from the dY images the dgrad
+// chain left in the gradient stash,
+//     d gamma(x) = dY_0 . W_0[:, 0:63] + dY_4 . W_4[:, 256:319]      d gamma(d) = dY_9 . W_cfc[:, 256:283]
+// One CTA per SM (cta_group::1), persistent over 128-point tiles.  The three B images (72 KB) stay resident in shared memory;
+// a tile's A images (dY_0, dY_4: K = 256; dY_9: K = 128; 160 KB) stream through a 4-slot ring of K = 64 slabs (16 KB, one
+// contiguous piece of a stash image) by bulk copies.  Both gamma(x) products chain into one N = 64 accumulator, gamma(d) into an
+// N = 32 one; two accumulator sets in TMEM, so the epilogue of a tile overlaps the MMAs of the next.  The epilogue (thread =
+// point) stages fp32 rows in shared memory and stores them coalesced.  1.25 KB read and 360 B written per point: HBM-bound.
+// Roles: warp 0 producer, warp 1 MMA issuer, warp 2 TMEM allocation, warps 4-7 epilogue.
+// =======================================================================================================
+struct DinputParams {
+    const uint8_t* packed; const uint8_t* dstash;
+    float* d_enc_pos; float* d_enc_dir;                 // [Q,63] / [Q,27], either may be null
+    int64_t Q, num_tiles;
+};
+constexpr int kDiSlab = 16384;
+constexpr int kDiStages = 4;
+constexpr int kDiSlabs = 10;                           // per tile: dY_0 x 4, dY_4 x 4, dY_9 x 2
+constexpr int kDiSmemRing = kDinImgBytes;
+constexpr int kDiSmemOut = kDiSmemRing + kDiStages * kDiSlab;
+constexpr int kDiOutFloats = TILE_M * (kPosDim + kDirDim);
+constexpr int kDiSmemBar = kDiSmemOut + kDiOutFloats * 4;
+constexpr int kDiSmemBytes = kDiSmemBar + 256;
+constexpr int kDiThreads = 256;
+constexpr uint32_t kDiTmemCols = 256;                  // accumulator set a at columns 128 a: gamma(x) [0, 64), gamma(d) [64, 96)
+static_assert(kDiSmemBytes <= 227 * 1024, "dinput shared memory");
+__host__ __device__ inline size_t dinput_slab_ofs(int s) {
+    return s < 4 ? dstash_ofs(0) + (size_t)s * kDiSlab : (s < 8 ? dstash_ofs(4) + (size_t)(s - 4) * kDiSlab : dstash_ofs(9) + (size_t)(s - 8) * kDiSlab);
+}
+
+__global__ void __launch_bounds__(kDiThreads, 1) field_dinput_kernel(const __grid_constant__ DinputParams p) {
+    extern __shared__ __align__(128) uint8_t smem[];
+    const uint32_t sbase = smem_u32(smem);
+    const int warp = threadIdx.x >> 5;
+    const uint32_t bar_full = sbase + kDiSmemBar, bar_empty = bar_full + 8 * kDiStages, bar_acc = bar_empty + 8 * kDiStages,
+                   bar_free = bar_acc + 16, bar_b = bar_free + 16;
+    volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(smem + kDiSmemBar + 8 * (2 * kDiStages + 5));
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < kDiStages; ++s) { mbar_init(bar_full + 8 * s, 1); mbar_init(bar_empty + 8 * s, 1); }
+        for (int a = 0; a < 2; ++a) { mbar_init(bar_acc + 8 * a, 1); mbar_init(bar_free + 8 * a, 128); }
+        mbar_init(bar_b, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    if (warp == 2) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32((const void*)tmem_slot)),
+                     "r"(kDiTmemCols)
+                     : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem_base = *tmem_slot;
+
+    if (warp == 0) {
+        if (elect_one()) {                                 // producer: B images once, then the A slabs of every tile
+            mbar_expect_tx(bar_b, kDinImgBytes);
+            bulk_g2s(sbase, p.packed + kDinImgOfs, kDinImgBytes, bar_b);
+            uint32_t stage = 0, round = 0;
+            for (int64_t tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
+                const uint8_t* ds = p.dstash + (size_t)tile * kDstashTile;
+                for (int s = 0; s < kDiSlabs; ++s) {
+                    mbar_wait(bar_empty + 8 * stage, (round & 1) ^ 1);
+                    mbar_expect_tx(bar_full + 8 * stage, kDiSlab);
+                    bulk_g2s(sbase + kDiSmemRing + stage * kDiSlab, ds + dinput_slab_ofs(s), kDiSlab, bar_full + 8 * stage);
+                    if (++stage == kDiStages) { stage = 0; ++round; }
+                }
+            }
+        }
+    } else if (warp == 1) {
+        if (elect_one()) {                                 // MMA issuer
+            // kind::f16, D = f32, A = B = bf16, both K-major, M = 128
+            constexpr uint32_t idesc_base = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(TILE_M >> 4) << 24);
+            constexpr uint32_t idesc_x = idesc_base | ((uint32_t)(64 >> 3) << 17), idesc_d = idesc_base | ((uint32_t)(32 >> 3) << 17);
+            const uint64_t ahi = desc_hi(2048, 128), bhi_x = desc_hi(64 * 16, 128), bhi_d = desc_hi(32 * 16, 128);
+            mbar_wait(bar_b, 0);
+            uint32_t stage = 0, round = 0, it = 0;
+            for (int64_t tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++it) {
+                const uint32_t acc = it & 1;
+                mbar_wait(bar_free + 8 * acc, ((it >> 1) & 1) ^ 1);          // the epilogue has drained this accumulator set
+                tc_fence_after();
+                const uint32_t d_x = tmem_base + acc * 128, d_d = d_x + 64;
+                for (int s = 0; s < kDiSlabs; ++s) {
+                    mbar_wait(bar_full + 8 * stage, round & 1);
+                    tc_fence_after();
+                    const uint32_t a0 = sbase + kDiSmemRing + stage * kDiSlab;
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) {                            // K = 16 steps of the slab
+                        const uint64_t ad = desc_at(ahi, a0 + j * 4096);
+                        if (s < 8) {
+                            const uint32_t k0 = (uint32_t)(s & 3) * 64 + j * 16;
+                            const uint32_t b = sbase + (s < 4 ? kDinPos0 : kDinPos4) + (k0 >> 3) * 1024;
+                            tc_mma(d_x, ad, desc_at(bhi_x, b), idesc_x, (s == 0 && j == 0) ? 0u : 1u);
+                        } else {
+                            const uint32_t k0 = (uint32_t)(s - 8) * 64 + j * 16;
+                            tc_mma(d_d, ad, desc_at(bhi_d, sbase + kDinDir + (k0 >> 3) * 512), idesc_d, (s == 8 && j == 0) ? 0u : 1u);
+                        }
+                    }
+                    tc_commit(bar_empty + 8 * stage);
+                    if (++stage == kDiStages) { stage = 0; ++round; }
+                }
+                tc_commit(bar_acc + 8 * acc);
+            }
+        }
+    } else if (warp >= 4) {
+        // epilogue: thread = accumulator row = point of the tile; rows staged in shared memory as the global [rows][63] / [rows][27]
+        // blocks (odd row strides: conflict-free), then copied out with consecutive threads on consecutive floats
+        const int r = (int)threadIdx.x - 128;
+        float* out_x = reinterpret_cast<float*>(smem + kDiSmemOut);
+        float* out_d = out_x + TILE_M * kPosDim;
+        uint32_t it = 0;
+        for (int64_t tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++it) {
+            const uint32_t acc = it & 1;
+            mbar_wait(bar_acc + 8 * acc, (it >> 1) & 1);
+            tc_fence_after();
+            const uint32_t trow = tmem_base + acc * 128 + ((uint32_t)((warp & 3) * 32) << 16);
+#pragma unroll 1
+            for (int c = 0; c < 6; ++c) {                                    // columns [0, 64) gamma(x), [64, 96) gamma(d)
+                uint32_t v[16];
+                tc_ld16(trow + 16 * c, v);
+                tc_wait_ld();
+                pin16(v);
+#pragma unroll
+                for (int j = 0; j < 16; ++j) {
+                    const int col = 16 * c + j;
+                    if (col < kPosDim) out_x[r * kPosDim + col] = __uint_as_float(v[j]);
+                    else if (col >= 64 && col < 64 + kDirDim) out_d[r * kDirDim + col - 64] = __uint_as_float(v[j]);
+                }
+            }
+            tc_fence_before();
+            mbar_arrive(bar_free + 8 * acc);
+            named_bar_sync(1, 128);
+            const int64_t rows = p.Q - tile * TILE_M < TILE_M ? p.Q - tile * TILE_M : TILE_M;
+            if (p.d_enc_pos) {
+                float* dst = p.d_enc_pos + tile * TILE_M * kPosDim;
+                for (int i = r; i < rows * kPosDim; i += 128) dst[i] = out_x[i];
+            }
+            if (p.d_enc_dir) {
+                float* dst = p.d_enc_dir + tile * TILE_M * kDirDim;
+                for (int i = r; i < rows * kDirDim; i += 128) dst[i] = out_d[i];
+            }
+            named_bar_sync(1, 128);                                          // staging area free for the next tile
+        }
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 2) {
+        tc_fence_after();
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kDiTmemCols) : "memory");
+    }
+}
+
+// B images of field_dinput_kernel: one thread per 16-byte row chunk (8 consecutive out features k of one in feature n)
+__device__ __forceinline__ void pack_tc_dinput(const float* __restrict__ params, uint8_t* __restrict__ out) {
+    const LayerDesc d0 = layer_desc(0), d4 = layer_desc(4), dc = layer_desc(10);
+    for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < 2 * 32 * 64 + 16 * 32; idx += gridDim.x * blockDim.x) {
+        int img = idx >> 11, rem = idx & 2047;
+        if (img > 2) img = 2;
+        if (img == 2) rem = idx - 2 * 2048;
+        const int rows = img < 2 ? 64 : 32, n = rem % rows, k8 = rem / rows;
+        const LayerDesc& d = img == 0 ? d0 : (img == 1 ? d4 : dc);
+        const int col = img == 0 ? n : kHidden + n, n_true = img < 2 ? kPosDim : kDirDim;
+        float x[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) x[j] = n < n_true ? params[d.w_off + (int64_t)(8 * k8 + j) * d.K + col] : 0.f;
+        const uint32_t base = img == 0 ? kDinPos0 : (img == 1 ? kDinPos4 : kDinDir);
+        *reinterpret_cast<uint4*>(out + kDinImgOfs + base + (size_t)(k8 * rows + n) * 16) =
+            make_uint4(pack_bf16(x[0], x[1]), pack_bf16(x[2], x[3]), pack_bf16(x[4], x[5]), pack_bf16(x[6], x[7]));
+    }
+}
+
 // transposed images for the dgrad chain
 __device__ __forceinline__ void pack_tc_transposed(const float* __restrict__ params, uint8_t* __restrict__ out, int m) {
     {
@@ -1555,7 +1731,8 @@ __device__ __forceinline__ void pack_tc_transposed(const float* __restrict__ par
     }
 }
 // one launch packs every image of up to four nets: blockIdx.y = forward layer 0..9 (bf16) | 10 + dgrad step 0..8 |
-// 19 + forward layer 0..9 (fp16 = split high halves) | 29 + forward layer 0..9 (split low halves), blockIdx.z = net
+// 19 input-gradient images | 20 + forward layer 0..9 (fp16 = split high halves) | 30 + forward layer 0..9 (split low halves),
+// blockIdx.z = net
 struct PackBatch { const float* params[4]; uint8_t* out[4]; uint64_t* counter; };
 __global__ void pack_tc_kernel(const PackBatch b) {
     // last kernel of a replayed training step: bump the device-side step counter (nothing else in this launch reads it, every
@@ -1565,8 +1742,9 @@ __global__ void pack_tc_kernel(const PackBatch b) {
     uint8_t* out = b.out[blockIdx.z];
     if (blockIdx.y < kNumMmaLayers) pack_tc_forward<0>(params, out, blockIdx.y);
     else if (blockIdx.y < kNumMmaLayers + kNumDgradLayers) pack_tc_transposed(params, out, blockIdx.y - kNumMmaLayers);
-    else if (blockIdx.y < 2 * kNumMmaLayers + kNumDgradLayers) pack_tc_forward<1>(params, out, blockIdx.y - kNumMmaLayers - kNumDgradLayers);
-    else pack_tc_forward<2>(params, out, blockIdx.y - 2 * kNumMmaLayers - kNumDgradLayers);
+    else if (blockIdx.y == kNumMmaLayers + kNumDgradLayers) pack_tc_dinput(params, out);
+    else if (blockIdx.y < 2 * kNumMmaLayers + kNumDgradLayers + 1) pack_tc_forward<1>(params, out, blockIdx.y - kNumMmaLayers - kNumDgradLayers - 1);
+    else pack_tc_forward<2>(params, out, blockIdx.y - 2 * kNumMmaLayers - kNumDgradLayers - 1);
 }
 
 }  // namespace tc
@@ -1585,8 +1763,8 @@ int tc_pack(const float* const* params, void* const* packed_bf16, int n_nets, bo
     tc::PackBatch b{};
     for (int i = 0; i < n_nets; ++i) { b.params[i] = params[i]; b.out[i] = reinterpret_cast<uint8_t*>(packed_bf16[i]); }
     b.counter = g_pack_counter;
-    // blockIdx.y: [0,19) = the training images (bf16 forward + transposed), [19,39) = the inference-only fp16 hi / lo images
-    const int ny = train_only ? tc::kNumMmaLayers + tc::kNumDgradLayers : 3 * tc::kNumMmaLayers + tc::kNumDgradLayers;
+    // blockIdx.y: [0,20) = the training images (bf16 forward + transposed + input-gradient), [20,40) = the inference-only fp16 hi / lo
+    const int ny = train_only ? tc::kNumMmaLayers + tc::kNumDgradLayers + 1 : 3 * tc::kNumMmaLayers + tc::kNumDgradLayers + 1;
     tc::pack_tc_kernel<<<dim3(32, ny, n_nets), 256, 0, st>>>(b);
     NSB_LAUNCH_CHECK("pack_tc_kernel");
     return NSB_OK;
@@ -1719,13 +1897,16 @@ int tc_field_fwd_enc(const float* enc_pos, const float* enc_dir, const void* pac
     return launch_fwd<true>(p, st);
 }
 
-// parameter grads (accumulated into the flat `grads`) from the forward stash in ws: dgrad chain -> wgrad -> head grads
-int tc_field_bwd(const float* d_raw, const void* packed, float* grads, void* ws, int64_t Q, cudaStream_t st) {
+// parameter grads (accumulated into the flat `grads`; none when it is null) and encoding grads (d_enc_pos / d_enc_dir, optional)
+// from the forward stash in ws: dgrad chain -> input-gradient products -> wgrad -> head grads
+int tc_field_bwd(const float* d_raw, const void* packed, float* grads, float* d_enc_pos, float* d_enc_dir, void* ws, int64_t Q,
+                 cudaStream_t st) {
     NSB_TRY(check_arch());
     static bool attr_set = false;
     if (!attr_set) {
         if (cudaFuncSetAttribute(tc::field_dgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kSmemBytes) != cudaSuccess ||
-            cudaFuncSetAttribute(tc::field_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kWgSmemBytes) != cudaSuccess)
+            cudaFuncSetAttribute(tc::field_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kWgSmemBytes) != cudaSuccess ||
+            cudaFuncSetAttribute(tc::field_dinput_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::kDiSmemBytes) != cudaSuccess)
             return check_launch("cudaFuncSetAttribute(bwd kernels)");
         attr_set = true;
     }
@@ -1740,6 +1921,15 @@ int tc_field_bwd(const float* d_raw, const void* packed, float* grads, void* ws,
     if (dgrid > num_sms()) dgrid -= 2;
     tc::field_dgrad_kernel<<<dgrid, tc::kThreads, tc::kSmemBytes, st>>>(dp);
     NSB_LAUNCH_CHECK("field_dgrad_kernel");
+    if (d_enc_pos || d_enc_dir) {
+        tc::DinputParams ip{};
+        ip.packed = reinterpret_cast<const uint8_t*>(packed); ip.dstash = ws_dstash(ws, Q);
+        ip.d_enc_pos = d_enc_pos; ip.d_enc_dir = d_enc_dir; ip.Q = Q; ip.num_tiles = tiles;
+        const int igrid = (int)(tiles < num_sms() ? tiles : num_sms());
+        tc::field_dinput_kernel<<<igrid, tc::kDiThreads, tc::kDiSmemBytes, st>>>(ip);
+        NSB_LAUNCH_CHECK("field_dinput_kernel");
+    }
+    if (!grads) return NSB_OK;
 
     tc::WgradParams wp{};
     wp.stash = ws_stash(ws); wp.dstash = ws_dstash(ws, Q); wp.d_raw = d_raw; wp.grads = grads; wp.num_tiles = tiles; wp.Q = Q;

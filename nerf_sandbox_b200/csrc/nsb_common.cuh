@@ -158,7 +158,8 @@ struct GemmArgs {
     const float* bias; int relu;        // FWD
     const float* mask; int64_t ldm;     // DGRAD: multiply by (mask > 0)
     const float* addend; int64_t ldadd; // DGRAD: += addend
-    int n_valid;                        // WGRAD: columns < n_valid are written
+    int n_valid;                        // WGRAD: columns < n_valid are written; DGRAD: when > 0, only columns < n_valid are
+                                        //   written (and addend read), with scalar accesses: C / addend of any leading dimension
     int64_t k_per_split;                // WGRAD: contraction rows per split
     float* colsum;                      // WGRAD on the tensor cores: += column sums of A (the bias gradient), or null
     const uint8_t* b_img;               // FWD / DGRAD on the tensor cores: pre-split term images of B (split_pack), or null
@@ -174,6 +175,7 @@ struct PackedLayout {
     size_t bf16_off;               // start of the bf16 image (layout owned by field_tc.cu)
     size_t bf16_bytes;
     size_t split_fwd[12], split_dgrad[12];   // bf16 term images of the weights for the fp32 mode's tensor-core GEMMs (field_split.cu)
+    size_t split_dinput[3];                   // ... and of the transposed input slices W_0[:, 0:63], W_4[:, 256:319], W_cfc[:, 256:283]
     size_t split_off, split_bytes;
     size_t total;
 };

@@ -9,6 +9,29 @@ import torch.nn as nn
 from . import _lib
 
 
+class _EncodeFn(torch.autograd.Function):
+    """gamma(x) with its backward (nsb_encode_bwd); used only when x requires grad."""
+
+    @staticmethod
+    def forward(ctx, x, D, L, include_input, out_dim):
+        xf = _lib.f32c(x).reshape(-1, D)
+        out = torch.empty((xf.shape[0], out_dim), device=x.device, dtype=torch.float32)
+        _lib.check(_lib.lib().nsb_encode(_lib.ptr(xf), _lib.ptr(out), xf.shape[0], D, L, int(include_input), _lib.stream()),
+                   "nsb_encode")
+        ctx.save_for_backward(xf)
+        ctx.cfg = (D, L, include_input, out_dim, x.shape, x.dtype)
+        return out.reshape(*x.shape[:-1], out_dim).to(x.dtype)
+
+    @staticmethod
+    def backward(ctx, g):
+        (xf,) = ctx.saved_tensors
+        D, L, include_input, out_dim, shape, dtype = ctx.cfg
+        gx = torch.empty_like(xf)
+        _lib.check(_lib.lib().nsb_encode_bwd(_lib.ptr(xf), _lib.ptr(_lib.f32c(g).reshape(-1, out_dim)), _lib.ptr(gx), xf.shape[0], D,
+                                             L, int(include_input), _lib.stream()), "nsb_encode_bwd")
+        return gx.reshape(shape).to(dtype), None, None, None, None
+
+
 class PositionalEncoder(nn.Module):
     """gamma(x) = [x (optional), sin(2^k x), cos(2^k x)], k = 0..num_freqs-1 (encoders.py:11-20)."""
 
@@ -35,6 +58,8 @@ class PositionalEncoder(nn.Module):
             raise NotImplementedError("nerf_sandbox_b200 encodes with freq_bands = 2^k, k=0..L-1, no 2*pi (vanilla path)")
         if x.shape[-1] != self.input_dims:
             raise RuntimeError(f"expected last dim {self.input_dims}, got {tuple(x.shape)}")
+        if torch.is_grad_enabled() and x.requires_grad:
+            return _EncodeFn.apply(x, self.input_dims, self.num_freqs, self.include_input, self.out_dim)
         xf = _lib.f32c(x).reshape(-1, self.input_dims)
         out = torch.empty((xf.shape[0], self.out_dim), device=x.device, dtype=torch.float32)
         _lib.check(_lib.lib().nsb_encode(_lib.ptr(xf), _lib.ptr(out), xf.shape[0], self.input_dims, self.num_freqs,

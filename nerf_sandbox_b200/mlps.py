@@ -63,14 +63,15 @@ class _Workspace:
 
 
 class _FieldEncFn(torch.autograd.Function):
-    """NeRF.forward on materialised encodings; grads w.r.t. the parameters only."""
+    """NeRF.forward on materialised encodings; grads w.r.t. the parameters and the two encodings."""
 
     @staticmethod
     def forward(ctx, nerf, grad_mode, enc_pos, enc_dir, *params):
         L = _lib.lib()
         ep, ed = _lib.f32c(enc_pos), _lib.f32c(enc_dir)
         Q = ep.shape[0]
-        need_grad = grad_mode and any(p.requires_grad for p in params)     # (grad mode is off inside forward)
+        need_grad = grad_mode and (enc_pos.requires_grad or enc_dir.requires_grad
+                                   or any(p.requires_grad for p in params))     # (grad mode is off inside forward)
         packed = nerf.packed()
         wsb = L.nsb_field_workspace_bytes(Q, nerf.mode, int(need_grad))
         ws = (torch.empty(wsb, dtype=torch.uint8, device=ep.device) if need_grad else nerf._ws.get(wsb, ep.device))
@@ -78,15 +79,25 @@ class _FieldEncFn(torch.autograd.Function):
         _lib.check(L.nsb_field_fwd_enc(_lib.ptr(ep), _lib.ptr(ed), _lib.ptr(packed), _lib.ptr(raw), _lib.ptr(ws), wsb, Q,
                                        nerf.mode, int(need_grad), _lib.stream()), "nsb_field_fwd_enc")
         ctx.nerf, ctx.ws, ctx.wsb, ctx.Q, ctx.packed = nerf, ws, wsb, Q, packed
+        ctx.enc_dtypes = (enc_pos.dtype, enc_dir.dtype)
         return raw
 
     @staticmethod
     def backward(ctx, d_raw):
         nerf = ctx.nerf
-        g = torch.zeros(_lib.N_PARAMS, device=d_raw.device, dtype=torch.float32)
-        _lib.check(_lib.lib().nsb_field_bwd(_lib.ptr(_lib.f32c(d_raw)), _lib.ptr(ctx.packed), _lib.ptr(g), _lib.ptr(ctx.ws),
-                                            ctx.wsb, ctx.Q, nerf.mode, _lib.stream()), "nsb_field_bwd")
-        return (None, None, None, None) + tuple(nerf.unflatten(g))
+        dev = d_raw.device
+        need_param = any(ctx.needs_input_grad[4:])
+        g = torch.zeros(_lib.N_PARAMS, device=dev, dtype=torch.float32) if need_param else None
+        d_ep = torch.empty((ctx.Q, nerf.enc_pos_dim), device=dev, dtype=torch.float32) if ctx.needs_input_grad[2] else None
+        d_ed = torch.empty((ctx.Q, nerf.enc_dir_dim), device=dev, dtype=torch.float32) if ctx.needs_input_grad[3] else None
+        if g is None and d_ep is None and d_ed is None:
+            return (None,) * len(ctx.needs_input_grad)
+        _lib.check(_lib.lib().nsb_field_bwd_ex(_lib.ptr(_lib.f32c(d_raw)), _lib.ptr(ctx.packed), _lib.ptr(g), _lib.ptr(d_ep),
+                                               _lib.ptr(d_ed), _lib.ptr(ctx.ws), ctx.wsb, ctx.Q, nerf.mode, _lib.stream()),
+                   "nsb_field_bwd_ex")
+        pgrads = tuple(nerf.unflatten(g)) if g is not None else (None,) * (len(ctx.needs_input_grad) - 4)
+        return (None, None, None if d_ep is None else d_ep.to(ctx.enc_dtypes[0]),
+                None if d_ed is None else d_ed.to(ctx.enc_dtypes[1])) + pgrads
 
 
 class NeRF(nn.Module):

@@ -72,14 +72,20 @@ def _is_fused_triplet(pos_enc, dir_enc, nerf) -> bool:
 
 
 class _FusedPassFn(torch.autograd.Function):
-    """rays + z -> (comp, weights, acc, depth); differentiable w.r.t. the NeRF parameters through comp."""
+    """rays + z -> (comp, weights, acc, depth); differentiable w.r.t. the NeRF parameters and the rays (rays_o, rays_d_unit,
+    viewdirs) through all four outputs.  No gradient w.r.t. z or ray_norm."""
 
     @staticmethod
-    def forward(ctx, nerf, grad_mode, o, d, z, rn, vd, flags, noise_std, noise, seed, *params):
+    def forward(ctx, nerf, grad_mode, rays_o, rays_d, z, rn, viewdirs, flags, noise_std, noise, seed, *params):
         L = _lib.lib()
         B, N = z.shape
         dev = z.device
-        need_grad = grad_mode and any(p.requires_grad for p in params)     # (grad mode is off inside forward)
+        o, d = _lib.f32c(rays_o), _lib.f32c(rays_d)
+        vd = None if viewdirs is None else _lib.f32c(viewdirs)
+        ray_grad = [t is not None and t.requires_grad for t in (rays_o, rays_d, viewdirs)]
+        need_param = grad_mode and any(p.requires_grad for p in params)     # (grad mode is off inside forward)
+        need_rays = grad_mode and any(ray_grad)
+        need_grad = need_param or need_rays
         packed = nerf.packed()
         wsb = L.nsb_field_workspace_bytes(B * N, nerf.mode, int(need_grad))
         ws = torch.empty(wsb, dtype=torch.uint8, device=dev) if need_grad else nerf._ws.get(wsb, dev)
@@ -95,26 +101,48 @@ class _FusedPassFn(torch.autograd.Function):
                                            _lib.ptr(comp), _lib.ptr(w), _lib.ptr(acc), _lib.ptr(depth), B, N, flags, seed, 0,
                                            _lib.stream()), "nsb_composite_raw_fwd")
         ctx.nerf, ctx.ws, ctx.wsb, ctx.packed = nerf, ws, wsb, packed
-        ctx.saved = (raw, z, rn, noise)
+        ctx.saved = (raw, z, rn, noise, o, d, vd)
         ctx.cfg = (B, N, flags, noise_std, seed)
-        # weights/acc/depth are used detached by every caller of the reference (trainer.py:928, render_utils.py:390)
-        ctx.mark_non_differentiable(w, acc, depth)
+        ctx.need_param = need_param
+        ctx.ray_meta = [(t.shape, t.dtype) if t is not None else None for t in (rays_o, rays_d, viewdirs)]
+        ctx.set_materialize_grads(False)
         return comp, w, acc, depth
 
     @staticmethod
     def backward(ctx, g_comp, g_w, g_acc, g_depth):
         L = _lib.lib()
         nerf = ctx.nerf
-        raw, z, rn, noise = ctx.saved
+        raw, z, rn, noise, o, d, vd = ctx.saved
         B, N, flags, noise_std, seed = ctx.cfg
+        n_params = len(ctx.needs_input_grad) - 11
+        want_o, want_d, want_vd = ctx.needs_input_grad[2], ctx.needs_input_grad[3], ctx.needs_input_grad[6]
+        if all(g is None for g in (g_comp, g_w, g_acc, g_depth)) or not (ctx.need_param or want_o or want_d or want_vd):
+            return (None,) * (11 + n_params)
         d_raw = torch.empty_like(raw)
-        _lib.check(L.nsb_composite_raw_bwd(_lib.ptr(raw), _lib.ptr(noise), noise_std, _lib.ptr(z), _lib.ptr(rn),
-                                           _lib.ptr(_lib.f32c(g_comp)), _lib.ptr(d_raw), B, N, flags, seed, 0,
-                                           _lib.stream()), "nsb_composite_raw_bwd")
-        g = torch.zeros(_lib.N_PARAMS, device=raw.device, dtype=torch.float32)
-        _lib.check(L.nsb_field_bwd(_lib.ptr(d_raw), _lib.ptr(ctx.packed), _lib.ptr(g), _lib.ptr(ctx.ws), ctx.wsb, B * N,
-                                   nerf.mode, _lib.stream()), "nsb_field_bwd")
-        return (None,) * 11 + tuple(nerf.unflatten(g))
+        g_acc = None if g_acc is None else _lib.f32c(g_acc).reshape(B)
+        g_depth = None if g_depth is None else _lib.f32c(g_depth).reshape(B)
+        _lib.check(L.nsb_composite_raw_bwd_ex(_lib.ptr(raw), _lib.ptr(noise), noise_std, _lib.ptr(z), _lib.ptr(rn),
+                                              _lib.ptr(_lib.f32c(g_comp)), _lib.ptr(_lib.f32c(g_w)), _lib.ptr(g_acc), _lib.ptr(g_depth),
+                                              _lib.ptr(d_raw), B, N, flags, seed, 0, _lib.stream()), "nsb_composite_raw_bwd_ex")
+        dev = raw.device
+        g = torch.zeros(_lib.N_PARAMS, device=dev, dtype=torch.float32) if ctx.need_param else None
+        rays = want_o or want_d or want_vd
+        d_ep = torch.empty((B * N, 63), device=dev, dtype=torch.float32) if rays else None
+        d_ed = torch.empty((B * N, 27), device=dev, dtype=torch.float32) if rays else None
+        _lib.check(L.nsb_field_bwd_ex(_lib.ptr(d_raw), _lib.ptr(ctx.packed), _lib.ptr(g), _lib.ptr(d_ep), _lib.ptr(d_ed),
+                                      _lib.ptr(ctx.ws), ctx.wsb, B * N, nerf.mode, _lib.stream()), "nsb_field_bwd_ex")
+        d_o = d_d = d_vd = None
+        if rays:
+            d_o = torch.empty((B, 3), device=dev) if want_o else None
+            # without explicit viewdirs the view-direction term belongs to rays_d (render_utils.py:218-222)
+            d_d = torch.empty((B, 3), device=dev) if want_d else None
+            d_vd = torch.empty((B, 3), device=dev) if want_vd else None
+            _lib.check(L.nsb_encode_bwd_rays(_lib.ptr(d_ep), _lib.ptr(d_ed), _lib.ptr(o), _lib.ptr(d), _lib.ptr(z), _lib.ptr(rn),
+                                             _lib.ptr(vd), _lib.ptr(d_o), _lib.ptr(d_d), _lib.ptr(d_vd), B, N, _lib.stream()),
+                       "nsb_encode_bwd_rays")
+        shaped = [None if (t is None or m is None) else t.reshape(m[0]).to(m[1]) for t, m in zip((d_o, d_d, d_vd), ctx.ray_meta)]
+        pgrads = tuple(nerf.unflatten(g)) if g is not None else (None,) * n_params
+        return (None, None, shaped[0], shaped[1], None, None, shaped[2]) + (None,) * 4 + pgrads
 
 
 def nerf_forward_pass(rays_o: torch.Tensor, rays_d_unit: torch.Tensor, z_vals: torch.Tensor, *, pos_enc, dir_enc, nerf,
@@ -138,17 +166,16 @@ def nerf_forward_pass(rays_o: torch.Tensor, rays_d_unit: torch.Tensor, z_vals: t
     if _is_fused_triplet(pos_enc, dir_enc, nerf) and act in ("relu", "softplus"):
         if act == "softplus":
             flags |= _lib.SIGMA_SOFTPLUS                      # render_utils.py:243-244, fused into the compositor kernels
-        o, d, z = _lib.f32c(rays_o), _lib.f32c(rays_d_unit), _lib.f32c(z_vals)
+        z = _lib.f32c(z_vals)
         rn = None if ray_norms is None else _lib.f32c(ray_norms).reshape(B)
-        vd = None if viewdirs_world_unit is None else _lib.f32c(viewdirs_world_unit)
         use_noise = training and raw_noise_std > 0.0
         if use_noise and raw_noise is None and _hooks.normal is not None:
             raw_noise = _hooks.normal(B * N, z.device)
         noise = _lib.f32c(raw_noise).reshape(-1) if (use_noise and raw_noise is not None) else None
         if seed is None:
             seed = int(torch.randint(0, 2 ** 62, (1,)).item()) if (use_noise and noise is None) else 0
-        comp, w, acc, depth = _FusedPassFn.apply(nerf, torch.is_grad_enabled(), o, d, z, rn, vd, flags, float(raw_noise_std) if use_noise else 0.0,
-                                                 noise, seed, *nerf.ordered_params())
+        comp, w, acc, depth = _FusedPassFn.apply(nerf, torch.is_grad_enabled(), rays_o, rays_d_unit, z, rn, viewdirs_world_unit, flags,
+                                                 float(raw_noise_std) if use_noise else 0.0, noise, seed, *nerf.ordered_params())
         return comp, w, acc, depth
 
     # ---- generic composition for foreign encoders / models (render_utils.py:209-276) ----
