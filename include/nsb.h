@@ -43,7 +43,7 @@ extern "C" {
 
 /* arithmetic mode of the field (encoder + MLP) kernels */
 #define NSB_MODE_FP32 0  /* fp32 activations / gradients in HBM, the 1e-4 parity mode: layer GEMMs on tcgen05 with
-                          * operands split into three bf16 terms (fp32-grade products), NSB_FP32_GEMM=ffma: CUDA cores */
+                          * operands split into three bf16 terms (fp32-grade products) */
 #define NSB_MODE_BF16 1  /* tcgen05 tensor cores, bf16 operands, fp32 accumulate in TMEM     */
 
 /* NeRF(63,27,8,256,skip_pos=4) -- models/mlps.py:41-134.  Flat parameter order is the reference's
@@ -150,7 +150,7 @@ int nsb_encode_bwd_rays(const float* d_enc_pos, const float* d_enc_dir, const fl
                         const float* ray_norm, const float* viewdirs, float* d_rays_o, float* d_rays_d, float* d_viewdirs,
                         int64_t B, int N, void* stream);
 
-/* Packed weights of one NeRF: fp32 padded rows for the FFMA path, and images in tcgen05 operand layout for the tensor
+/* Packed weights of one NeRF: fp32 padded rows (heads and biases of the fp32 mode), and images in tcgen05 operand layout for the tensor
  * paths -- bf16 (training forward), transposed bf16 (dgrad), fp16 (inference forward) and the fp16 low halves of the
  * split used by the fp32-accurate inference forward, and bf16 term images (w = w0 + w1 + w2) of every weight matrix, plain
  * and transposed, for the fp32 mode's tensor-core layer GEMMs.  Sizes in bytes. */

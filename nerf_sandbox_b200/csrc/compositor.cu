@@ -4,7 +4,6 @@
 // The exclusive cumprod transmittance is a multiplicative warp scan carried across 32-sample chunks;
 // rgb/depth/acc reductions ride the same pass.  The backward recomputes T (never reads it from HBM),
 // stages alpha/T per warp in shared memory and walks the ray in reverse with a suffix-sum scan.
-#include <cstdlib>
 #include "nsb_common.cuh"
 
 namespace nsb {
@@ -266,8 +265,7 @@ constexpr int kRunWarps = 4;
 // One warp per ray up to 192 samples (R <= 6); above, 2-4 warps per ray with R = 4..6 each (7, 8 beyond 768): measured, the R = 8
 // single-warp kernels (120-160 registers) stream at 0.53-0.58 of the HBM roof where R <= 6 reaches 0.7-0.86.
 constexpr int kRunOneWarpMaxN = 192;
-// NSB_K3_STRIDED=1 forces the strided kernels for every N (A/B timing and debugging)
-static const int kRunMaxN = [] { const char* e = getenv("NSB_K3_STRIDED"); return (e && e[0] == '1') ? 0 : 1024; }();   // up to 4 warps per ray
+constexpr int kRunMaxN = 1024;                  // up to 4 warps per ray
 
 // 1 / (1 + 2^(-x log2 e)): FMUL + MUFU.EX2 + FADD + MUFU.RCP (relative error ~4e-7; saturates to 0 / 1, NaN propagates)
 __device__ __forceinline__ float fast_sigmoid(float x) { return rcp_approx(1.0f + ex2_approx(-1.4426950408889634f * x)); }

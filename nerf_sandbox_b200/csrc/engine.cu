@@ -35,9 +35,9 @@ int num_sms() {
 // field_fp32.cu
 size_t fp32_workspace_bytes(int64_t Q, int stash);
 int pack_fp32(const float* params, void* packed, cudaStream_t st);
-int fp32_prepare_rays(const float*, const float*, const float*, const float*, const float*, void*, int64_t, int, int, cudaStream_t);
-int fp32_prepare_enc(const float*, const float*, void*, int64_t, int, cudaStream_t);
-int fp32_mlp_fwd(const void* packed, float* raw, void* ws, int64_t Q, int stash, cudaStream_t st);
+int fp32_prepare_rays(const float*, const float*, const float*, const float*, const float*, void*, int64_t, int, cudaStream_t);
+int fp32_prepare_enc(const float*, const float*, void*, int64_t, cudaStream_t);
+int fp32_mlp_fwd(const void* packed, float* raw, void* ws, int64_t Q, cudaStream_t st);
 int fp32_mlp_bwd(const float* d_raw, const void* packed, float* grads, float* d_enc_pos, float* d_enc_dir, void* ws, int64_t Q,
                  cudaStream_t st);
 // field_tc.cu
@@ -53,15 +53,11 @@ int tc_field_fwd_enc(const float* enc_pos, const float* enc_dir, const void* pac
 int tc_field_bwd(const float* d_raw, const void* packed, float* grads, float* d_enc_pos, float* d_enc_dir, void* ws, int64_t Q,
                  cudaStream_t st);
 
+// The fp32 parity mode's INFERENCE forward (no stash) runs on the tensor cores with fp16-split operands (field_tc.cu:
+// field_fwd_split_kernel, fp32-accurate).
 int tc_field_fwd_rays_split(const float*, const float*, const float*, const float*, const float*, const void* packed, float* raw,
                             int64_t B, int N, cudaStream_t st);
 int tc_field_fwd_enc_split(const float* enc_pos, const float* enc_dir, const void* packed, float* raw, int64_t Q, cudaStream_t st);
-// The fp32 parity mode's INFERENCE forward (no stash) runs on the tensor cores with fp16-split operands (field_tc.cu:
-// field_fwd_split_kernel, fp32-accurate); NSB_FP32_EVAL=ffma keeps it on the FFMA kernels (A/B and debugging).
-static bool fp32_eval_on_tc() {
-    static const bool on = [] { const char* e = getenv("NSB_FP32_EVAL"); return !(e && e[0] == 'f'); }();
-    return on;
-}
 
 int composite_raw_fwd_at(const float* raw, const float* noise, float noise_std, const float* z, const float* ray_norm, float* comp,
                          float* weights, float* acc, float* depth, int64_t B, int N, uint32_t flags, uint64_t seed, uint64_t offset,
@@ -104,7 +100,7 @@ extern "C" int nsb_pack_weights_batch(const float* const* params, void* const* p
     }
     // one launch for all nets and images; the fp32 mode needs the tensor-core images too (split-operand inference forward)
     if (mode != NSB_MODE_FP32) NSB_TRY(tc_pack(params, bf16, n_nets, train_only, as_stream(stream)));
-    else if (fp32_eval_on_tc() && !train_only) NSB_TRY(tc_pack(params, bf16, n_nets, false, as_stream(stream)));
+    else if (!train_only) NSB_TRY(tc_pack(params, bf16, n_nets, false, as_stream(stream)));
     return NSB_OK;
 }
 
@@ -122,10 +118,10 @@ extern "C" int nsb_field_fwd_enc(const float* enc_pos, const float* enc_dir, con
     if (mode == NSB_MODE_BF16)
         return tc_field_fwd_enc(enc_pos, enc_dir, reinterpret_cast<const char*>(packed) + packed_layout().bf16_off, raw,
                                 ws, Q, stash, as_stream(stream));
-    if (!stash && fp32_eval_on_tc())
+    if (!stash)
         return tc_field_fwd_enc_split(enc_pos, enc_dir, reinterpret_cast<const char*>(packed) + packed_layout().bf16_off, raw, Q, as_stream(stream));
-    NSB_TRY(fp32_prepare_enc(enc_pos, enc_dir, ws, Q, stash, as_stream(stream)));
-    return fp32_mlp_fwd(packed, raw, ws, Q, stash, as_stream(stream));
+    NSB_TRY(fp32_prepare_enc(enc_pos, enc_dir, ws, Q, as_stream(stream)));
+    return fp32_mlp_fwd(packed, raw, ws, Q, as_stream(stream));
 }
 
 extern "C" int nsb_field_fwd_rays(const float* rays_o, const float* rays_d, const float* z, const float* ray_norm,
@@ -139,11 +135,11 @@ extern "C" int nsb_field_fwd_rays(const float* rays_o, const float* rays_d, cons
         return tc_field_fwd_rays(rays_o, rays_d, z, ray_norm, viewdirs,
                                  reinterpret_cast<const char*>(packed) + packed_layout().bf16_off, raw, ws, B, N, stash,
                                  as_stream(stream));
-    if (!stash && fp32_eval_on_tc())
+    if (!stash)
         return tc_field_fwd_rays_split(rays_o, rays_d, z, ray_norm, viewdirs, reinterpret_cast<const char*>(packed) + packed_layout().bf16_off, raw,
                                        B, N, as_stream(stream));
-    NSB_TRY(fp32_prepare_rays(rays_o, rays_d, z, ray_norm, viewdirs, ws, B, N, stash, as_stream(stream)));
-    return fp32_mlp_fwd(packed, raw, ws, Q, stash, as_stream(stream));
+    NSB_TRY(fp32_prepare_rays(rays_o, rays_d, z, ray_norm, viewdirs, ws, B, N, as_stream(stream)));
+    return fp32_mlp_fwd(packed, raw, ws, Q, as_stream(stream));
 }
 
 extern "C" int nsb_field_bwd_ex(const float* d_raw, const void* packed, float* grads, float* d_enc_pos, float* d_enc_dir, void* ws,

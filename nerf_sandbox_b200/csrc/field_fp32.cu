@@ -1,9 +1,9 @@
-// K1 (fp32 mode) -- positional encoder + NeRF MLP on CUDA cores, fp32 end to end.
-// This is the 1e-4 parity mode of the field: layer-by-layer register-tiled SGEMMs (128x128x16 tiles,
-// 8x8 micro-tiles, FFMA) with the bias/ReLU/mask epilogues fused, concat-free activation layout
+// K1 (fp32 mode) -- positional encoder + NeRF MLP with fp32 activations and gradients end to end.
+// This is the 1e-4 parity mode of the field for training: one GEMM per layer and role on the tensor cores with bf16-split
+// operands (field_split.cu) and the bias/ReLU/mask epilogues fused, concat-free activation layout
 // (layer 3 writes straight into the [h | gamma(x)] buffer of the skip layer, `feature` into the
 // [feat | gamma(d)] buffer of color_fc), dedicated warp-per-point kernels for the N=1/N=3 heads.
-// The tensor-core mode lives in field_tc.cu.
+// The inference forward (no stash) and the bf16 mode live in field_tc.cu.
 #include <cstdio>
 #include <cstdlib>
 #include "nsb_common.cuh"
@@ -21,7 +21,7 @@ struct Fp32Ws {
     size_t bytes;
 };
 
-static Fp32Ws carve_fp32(void* base, int64_t Q, int stash) {
+static Fp32Ws carve_fp32(void* base, int64_t Q) {
     Fp32Ws w;
     char* p = reinterpret_cast<char*>(base);
     size_t off = 0;
@@ -31,26 +31,23 @@ static Fp32Ws carve_fp32(void* base, int64_t Q, int stash) {
         return r;
     };
     w.X0 = take(kPosPad); w.X4 = take(kSkipPad); w.XC = take(kColorPad); w.C = take(kColorHidden);
-    if (stash) {
-        for (int l = 0; l < 8; ++l) {
-            if (l == 3) { w.out[l] = w.X4; w.out_ld[l] = kSkipPad; }
-            else { w.out[l] = take(kHidden); w.out_ld[l] = kHidden; }
-        }
-        w.dA = take(kHidden); w.dB = take(kHidden); w.dC = take(kColorHidden);
-    } else {
-        float* Ha = take(kHidden); float* Hb = take(kHidden);
-        for (int l = 0; l < 8; ++l) {
-            if (l == 3) { w.out[l] = w.X4; w.out_ld[l] = kSkipPad; }
-            else { w.out[l] = (l % 2 == 0) ? Ha : Hb; w.out_ld[l] = kHidden; }
-        }
-        // l=7 -> Hb, l=6 -> Ha, l=5 -> Hb, l=4 -> Ha: consecutive layers never alias
-        w.dA = w.dB = w.dC = nullptr;
+    for (int l = 0; l < 8; ++l) {
+        if (l == 3) { w.out[l] = w.X4; w.out_ld[l] = kSkipPad; }
+        else { w.out[l] = take(kHidden); w.out_ld[l] = kHidden; }
     }
+    w.dA = take(kHidden); w.dB = take(kHidden); w.dC = take(kColorHidden);
     w.bytes = off;
     return w;
 }
 
-size_t fp32_workspace_bytes(int64_t Q, int stash) { return carve_fp32(nullptr, Q, stash).bytes; }
+// Without a stash (inference) the forward is field_tc.cu's fp16-split kernel, which uses no workspace.  The size reported
+// for that case stays at the input buffers plus two hidden-layer buffers: nsb_field_workspace_bytes and
+// nsb_render_workspace_bytes are part of the C ABI.
+size_t fp32_workspace_bytes(int64_t Q, int stash) {
+    if (stash) return carve_fp32(nullptr, Q).bytes;
+    auto buf = [&](int64_t floats_per_pt) { return align_up((size_t)Q * floats_per_pt * sizeof(float), 256); };
+    return buf(kPosPad) + buf(kSkipPad) + buf(kColorPad) + buf(kColorHidden) + 2 * buf(kHidden);
+}
 
 // ---------------------------------------------------------------------------------------------------
 // encoders
@@ -247,140 +244,6 @@ __global__ void prepare_from_enc_kernel(const float* __restrict__ enc_pos, const
 }
 
 // ---------------------------------------------------------------------------------------------------
-// SGEMM  C[m,n] = sum_k A(m,k) * B(n,k)
-// ---------------------------------------------------------------------------------------------------
-constexpr int BM = 128, BN = 128, BK = 16, PITCH = 132;
-template <bool T>
-__device__ __forceinline__ void load_tile(const float* __restrict__ P, int64_t ld, int64_t row0, int64_t rows,
-                                          int64_t k0, int64_t kend, int tid, float4 (&reg)[2]) {
-    // T=false: P[(row0+r)*ld + k0+kk], float4 along k.   T=true: P[(k0+kk)*ld + row0+r], float4 along r.
-#pragma unroll
-    for (int i = 0; i < 2; ++i) {
-        const int idx = tid + i * 256;
-        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (!T) {
-            const int r = idx >> 2, kq = idx & 3;
-            if (row0 + r < rows && k0 + kq * 4 < kend) v = __ldg(reinterpret_cast<const float4*>(P + (row0 + r) * ld + k0 + kq * 4));
-        } else {
-            const int kk = idx >> 5, rq = idx & 31;
-            if (k0 + kk < kend && row0 + rq * 4 < rows) v = __ldg(reinterpret_cast<const float4*>(P + (k0 + kk) * ld + row0 + rq * 4));
-        }
-        reg[i] = v;
-    }
-}
-template <bool T>
-__device__ __forceinline__ void store_tile(float (*S)[PITCH], int tid, const float4 (&reg)[2]) {
-#pragma unroll
-    for (int i = 0; i < 2; ++i) {
-        const int idx = tid + i * 256;
-        if (!T) {
-            const int r = idx >> 2, kq = idx & 3;
-            S[kq * 4 + 0][r] = reg[i].x; S[kq * 4 + 1][r] = reg[i].y; S[kq * 4 + 2][r] = reg[i].z; S[kq * 4 + 3][r] = reg[i].w;
-        } else {
-            const int kk = idx >> 5, rq = idx & 31;
-            *reinterpret_cast<float4*>(&S[kk][rq * 4]) = reg[i];
-        }
-    }
-}
-
-template <bool AT, bool BT, int EPI>
-__global__ void __launch_bounds__(256) sgemm_kernel(GemmArgs g) {
-    __shared__ __align__(16) float As[BK][PITCH];
-    __shared__ __align__(16) float Bs[BK][PITCH];
-    const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
-    const int64_t m0 = (int64_t)blockIdx.x * BM, n0 = (int64_t)blockIdx.y * BN;
-    int64_t kbeg = 0, kend = g.Kdim;
-    if (EPI == EPI_WGRAD) {
-        kbeg = (int64_t)blockIdx.z * g.k_per_split;
-        kend = kbeg + g.k_per_split < g.Kdim ? kbeg + g.k_per_split : g.Kdim;
-        if (kbeg >= kend) return;
-    }
-    float acc[8][8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i)
-#pragma unroll
-        for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
-    float4 ra[2], rb[2];
-    load_tile<AT>(g.A, g.lda, m0, g.Mdim, kbeg, kend, tid, ra);
-    load_tile<BT>(g.B, g.ldb, n0, g.Ndim, kbeg, kend, tid, rb);
-    store_tile<AT>(As, tid, ra); store_tile<BT>(Bs, tid, rb);
-    __syncthreads();
-    for (int64_t k0 = kbeg; k0 < kend; k0 += BK) {
-        const bool more = k0 + BK < kend;
-        if (more) {
-            load_tile<AT>(g.A, g.lda, m0, g.Mdim, k0 + BK, kend, tid, ra);
-            load_tile<BT>(g.B, g.ldb, n0, g.Ndim, k0 + BK, kend, tid, rb);
-        }
-#pragma unroll
-        for (int kk = 0; kk < BK; ++kk) {
-            const float4 a0 = *reinterpret_cast<const float4*>(&As[kk][ty * 4]);
-            const float4 a1 = *reinterpret_cast<const float4*>(&As[kk][64 + ty * 4]);
-            const float4 b0 = *reinterpret_cast<const float4*>(&Bs[kk][tx * 4]);
-            const float4 b1 = *reinterpret_cast<const float4*>(&Bs[kk][64 + tx * 4]);
-            const float av[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
-            const float bv[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
-#pragma unroll
-            for (int i = 0; i < 8; ++i)
-#pragma unroll
-                for (int j = 0; j < 8; ++j) acc[i][j] = fmaf(av[i], bv[j], acc[i][j]);
-        }
-        __syncthreads();
-        if (more) {
-            store_tile<AT>(As, tid, ra); store_tile<BT>(Bs, tid, rb);
-            __syncthreads();
-        }
-    }
-    // epilogue
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        const int64_t m = m0 + (i < 4 ? ty * 4 + i : 64 + ty * 4 + (i - 4));
-        if (m >= g.Mdim) continue;
-#pragma unroll
-        for (int jh = 0; jh < 2; ++jh) {
-            const int64_t n = n0 + jh * 64 + tx * 4;
-            if (n >= g.Ndim) continue;
-            float v[4] = {acc[i][jh * 4 + 0], acc[i][jh * 4 + 1], acc[i][jh * 4 + 2], acc[i][jh * 4 + 3]};
-            if (EPI == EPI_FWD) {
-                const float4 bb = __ldg(reinterpret_cast<const float4*>(g.bias + n));
-                v[0] += bb.x; v[1] += bb.y; v[2] += bb.z; v[3] += bb.w;
-                if (g.relu) { v[0] = fmaxf(v[0], 0.f); v[1] = fmaxf(v[1], 0.f); v[2] = fmaxf(v[2], 0.f); v[3] = fmaxf(v[3], 0.f); }
-                *reinterpret_cast<float4*>(g.C + m * g.ldc + n) = make_float4(v[0], v[1], v[2], v[3]);
-            } else if (EPI == EPI_DGRAD && g.n_valid > 0) {
-#pragma unroll
-                for (int j = 0; j < 4; ++j)
-                    if (n + j < g.n_valid) g.C[m * g.ldc + n + j] = v[j] + (g.addend ? g.addend[m * g.ldadd + n + j] : 0.f);
-            } else if (EPI == EPI_DGRAD) {
-                if (g.addend) {
-                    const float4 ad = *reinterpret_cast<const float4*>(g.addend + m * g.ldadd + n);
-                    v[0] += ad.x; v[1] += ad.y; v[2] += ad.z; v[3] += ad.w;
-                }
-                if (g.mask) {
-                    const float4 mk = __ldg(reinterpret_cast<const float4*>(g.mask + m * g.ldm + n));
-                    v[0] = mk.x > 0.f ? v[0] : 0.f; v[1] = mk.y > 0.f ? v[1] : 0.f;
-                    v[2] = mk.z > 0.f ? v[2] : 0.f; v[3] = mk.w > 0.f ? v[3] : 0.f;
-                }
-                *reinterpret_cast<float4*>(g.C + m * g.ldc + n) = make_float4(v[0], v[1], v[2], v[3]);
-            } else {
-#pragma unroll
-                for (int j = 0; j < 4; ++j)
-                    if (n + j < g.n_valid) atomicAdd(g.C + m * g.ldc + n + j, v[j]);
-            }
-        }
-    }
-}
-
-// column sums for the bias gradients: out[n] += sum_m Y[m*ld + n]
-__global__ void colsum_kernel(const float* __restrict__ Y, int64_t ld, float* __restrict__ out, int64_t Q, int Ncols,
-                              int64_t rows_per_block) {
-    const int col = threadIdx.x % Ncols, sub = threadIdx.x / Ncols, nsub = blockDim.x / Ncols;
-    const int64_t r0 = (int64_t)blockIdx.x * rows_per_block;
-    const int64_t r1 = r0 + rows_per_block < Q ? r0 + rows_per_block : Q;
-    float s = 0.f;
-    for (int64_t r = r0 + sub; r < r1; r += nsub) s += Y[r * ld + col];
-    atomicAdd(out + col, s);
-}
-
-// ---------------------------------------------------------------------------------------------------
 // heads: sigma_out (256->1) and color_out (128->3), warp per point
 // ---------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
@@ -533,49 +396,31 @@ static inline const float* PB(const void* packed, const PackedLayout& L, int l) 
 }
 static inline const uint8_t* IMG(const void* packed, size_t off) { return reinterpret_cast<const uint8_t*>(packed) + off; }
 
-// The layer GEMMs run on the tensor cores with bf16-split operands (field_split.cu); NSB_FP32_GEMM=ffma keeps the FFMA tiles
-// of this file (the round-1 path, kept as the cross-check the split path is measured against).
-static bool gemm_on_tc() {
-    static const bool tc = [] { const char* e = getenv("NSB_FP32_GEMM"); return !(e && e[0] == 'f'); }();
-    return tc;
-}
-
-static int gemm_fwd(const float* X, int64_t ldx, const float* W, const uint8_t* w_img, int Kpad, const float* bias, float* Y, int64_t ldy,
+// The layer GEMMs run on the tensor cores with bf16-split operands (field_split.cu).  The forward, dgrad and input-gradient
+// GEMMs take the weights (their B operand) from the term images split_pack writes into the packed weights.
+static int gemm_fwd(const float* X, int64_t ldx, const uint8_t* w_img, int Kpad, const float* bias, float* Y, int64_t ldy,
                     int64_t Q, int N, int relu, cudaStream_t st) {
     GemmArgs g{};
-    g.A = X; g.lda = ldx; g.B = W; g.ldb = Kpad; g.C = Y; g.ldc = ldy; g.Mdim = Q; g.Ndim = N; g.Kdim = Kpad;
+    g.A = X; g.lda = ldx; g.C = Y; g.ldc = ldy; g.Mdim = Q; g.Ndim = N; g.Kdim = Kpad;
     g.bias = bias; g.relu = relu; g.b_img = w_img;
-    if (gemm_on_tc()) return split_gemm(g, EPI_FWD, st);
-    dim3 grid((unsigned)cdiv(Q, BM), (unsigned)cdiv(N, BN), 1);
-    sgemm_kernel<false, false, EPI_FWD><<<grid, 256, 0, st>>>(g);
-    NSB_LAUNCH_CHECK("sgemm_fwd");
-    return NSB_OK;
+    return split_gemm(g, EPI_FWD, st);
 }
-// dX[Q, n_in] = dY[Q, n_out] . W[n_out, ldw]  (first n_in columns), (+addend) (*mask)
-static int gemm_dgrad(const float* dY, int64_t ldy, const float* W, const uint8_t* w_img, int ldw, float* dX, int64_t ldx, int64_t Q,
-                      int n_out, int n_in, const float* mask, int64_t ldm, const float* addend, int64_t ldadd,
-                      cudaStream_t st) {
+// dX[Q, n_in] = dY[Q, n_out] . W[n_out, :n_in], (+addend) (*mask)
+static int gemm_dgrad(const float* dY, int64_t ldy, const uint8_t* w_img, float* dX, int64_t ldx, int64_t Q, int n_out, int n_in,
+                      const float* mask, int64_t ldm, const float* addend, int64_t ldadd, cudaStream_t st) {
     GemmArgs g{};
-    g.A = dY; g.lda = ldy; g.B = W; g.ldb = ldw; g.C = dX; g.ldc = ldx; g.Mdim = Q; g.Ndim = n_in; g.Kdim = n_out;
+    g.A = dY; g.lda = ldy; g.C = dX; g.ldc = ldx; g.Mdim = Q; g.Ndim = n_in; g.Kdim = n_out;
     g.mask = mask; g.ldm = ldm; g.addend = addend; g.ldadd = ldadd; g.b_img = w_img;
-    if (gemm_on_tc()) return split_gemm(g, EPI_DGRAD, st);
-    dim3 grid((unsigned)cdiv(Q, BM), (unsigned)cdiv(n_in, BN), 1);
-    sgemm_kernel<false, true, EPI_DGRAD><<<grid, 256, 0, st>>>(g);
-    NSB_LAUNCH_CHECK("sgemm_dgrad");
-    return NSB_OK;
+    return split_gemm(g, EPI_DGRAD, st);
 }
-// Input gradient: dE[Q, n_valid] (row stride lde, any) = dY[Q, n_out] . W[n_out, ldw] (n_in columns from W, n_in a multiple of 16
-// covering n_valid; the padding columns of W are zero) (+ addend, same layout as dE)
-static int gemm_dinput(const float* dY, int64_t ldy, const float* W, const uint8_t* w_img, int ldw, float* dE, int64_t lde, int64_t Q,
-                       int n_out, int n_in, int n_valid, const float* addend, cudaStream_t st) {
+// Input gradient: dE[Q, n_valid] (row stride lde, any) = dY[Q, n_out] . W_slice[n_out, n_in] (n_in a multiple of 16 covering
+// n_valid; the image's padding columns are zero) (+ addend, same layout as dE)
+static int gemm_dinput(const float* dY, int64_t ldy, const uint8_t* w_img, float* dE, int64_t lde, int64_t Q, int n_out, int n_in,
+                       int n_valid, const float* addend, cudaStream_t st) {
     GemmArgs g{};
-    g.A = dY; g.lda = ldy; g.B = W; g.ldb = ldw; g.C = dE; g.ldc = lde; g.Mdim = Q; g.Ndim = n_in; g.Kdim = n_out;
+    g.A = dY; g.lda = ldy; g.C = dE; g.ldc = lde; g.Mdim = Q; g.Ndim = n_in; g.Kdim = n_out;
     g.addend = addend; g.ldadd = lde; g.n_valid = n_valid; g.b_img = w_img;
-    if (gemm_on_tc()) return split_gemm(g, EPI_DGRAD, st);
-    dim3 grid((unsigned)cdiv(Q, BM), (unsigned)cdiv(n_in, BN), 1);
-    sgemm_kernel<false, true, EPI_DGRAD><<<grid, 256, 0, st>>>(g);
-    NSB_LAUNCH_CHECK("sgemm_dinput");
-    return NSB_OK;
+    return split_gemm(g, EPI_DGRAD, st);
 }
 // gW[n_out, K] += dY[Q, n_out]^T . X[Q, Kpad] ; gb[n_out] += colsum(dY)
 static int gemm_wgrad(const float* dY, int64_t ldy, const float* X, int64_t ldx, float* gW, float* gb, int64_t Q,
@@ -583,28 +428,8 @@ static int gemm_wgrad(const float* dY, int64_t ldy, const float* X, int64_t ldx,
     GemmArgs g{};
     g.A = dY; g.lda = ldy; g.B = X; g.ldb = ldx; g.C = gW; g.ldc = K; g.Mdim = n_out; g.Ndim = Kpad; g.Kdim = Q;
     g.n_valid = K;
-    if (gemm_on_tc()) {
-        g.colsum = gb;                      // the bias gradient rides along (the kernel sees every dY element anyway)
-        return split_gemm(g, EPI_WGRAD, st);
-    } else {
-        const int tiles = (int)(cdiv(n_out, BM) * cdiv(Kpad, BN));
-        int64_t splits = (int64_t)num_sms() * 2 / tiles;
-        if (splits < 1) splits = 1;
-        int64_t kps = cdiv(cdiv(Q, splits), BK) * BK;
-        if (kps < 256) kps = 256;
-        splits = cdiv(Q, kps);
-        g.k_per_split = kps;
-        dim3 grid((unsigned)cdiv(n_out, BM), (unsigned)cdiv(Kpad, BN), (unsigned)splits);
-        sgemm_kernel<true, true, EPI_WGRAD><<<grid, 256, 0, st>>>(g);
-        NSB_LAUNCH_CHECK("sgemm_wgrad");
-    }
-    // enough blocks to fill the GPU (4 per SM): at 2048 rows per block a 196,608-point pass launched 96 blocks -- less than
-    // one wave -- and the bias grads cost more than any SGEMM of the step
-    int64_t rpb = cdiv(Q, (int64_t)num_sms() * 4);
-    rpb = rpb < 64 ? 64 : rpb;
-    colsum_kernel<<<(unsigned)cdiv(Q, rpb), 256, 0, st>>>(dY, ldy, gb, Q, n_out, rpb);
-    NSB_LAUNCH_CHECK("colsum_kernel");
-    return NSB_OK;
+    g.colsum = gb;                      // the bias gradient rides along (the kernel sees every dY element anyway)
+    return split_gemm(g, EPI_WGRAD, st);
 }
 
 static int elem_grid(int64_t total) {
@@ -613,33 +438,33 @@ static int elem_grid(int64_t total) {
 }
 
 int fp32_prepare_rays(const float* o, const float* d, const float* z, const float* rn, const float* vd, void* ws,
-                      int64_t B, int N, int stash, cudaStream_t st) {
-    Fp32Ws w = carve_fp32(ws, B * (int64_t)N, stash);
+                      int64_t B, int N, cudaStream_t st) {
+    Fp32Ws w = carve_fp32(ws, B * (int64_t)N);
     prepare_from_rays_kernel<<<elem_grid(B * (int64_t)N * 16), 256, 0, st>>>(o, d, z, rn, vd, w.X0, w.X4, w.XC, B, N);
     NSB_LAUNCH_CHECK("prepare_from_rays_kernel");
     return NSB_OK;
 }
-int fp32_prepare_enc(const float* ep, const float* ed, void* ws, int64_t Q, int stash, cudaStream_t st) {
-    Fp32Ws w = carve_fp32(ws, Q, stash);
+int fp32_prepare_enc(const float* ep, const float* ed, void* ws, int64_t Q, cudaStream_t st) {
+    Fp32Ws w = carve_fp32(ws, Q);
     prepare_from_enc_kernel<<<elem_grid(Q * 96), 256, 0, st>>>(ep, ed, w.X0, w.X4, w.XC, Q);
     NSB_LAUNCH_CHECK("prepare_from_enc_kernel");
     return NSB_OK;
 }
 
 // mlps.py:221-278 on the prepared buffers
-int fp32_mlp_fwd(const void* packed, float* raw, void* ws, int64_t Q, int stash, cudaStream_t st) {
+int fp32_mlp_fwd(const void* packed, float* raw, void* ws, int64_t Q, cudaStream_t st) {
     const PackedLayout L = packed_layout();
-    Fp32Ws w = carve_fp32(ws, Q, stash);
+    Fp32Ws w = carve_fp32(ws, Q);
     const float* in = w.X0; int64_t ldin = kPosPad;
     for (int l = 0; l < 8; ++l) {
         const LayerDesc d = layer_desc(l);
         if (l == 4) { in = w.X4; ldin = kSkipPad; }
-        NSB_TRY(gemm_fwd(in, ldin, PW(packed, L, l), IMG(packed, L.split_fwd[l]), d.Kpad, PB(packed, L, l), w.out[l], w.out_ld[l], Q, 256, 1, st));
+        NSB_TRY(gemm_fwd(in, ldin, IMG(packed, L.split_fwd[l]), d.Kpad, PB(packed, L, l), w.out[l], w.out_ld[l], Q, 256, 1, st));
         in = w.out[l]; ldin = w.out_ld[l];
     }
     const float* H8 = w.out[7];
-    NSB_TRY(gemm_fwd(H8, kHidden, PW(packed, L, 8), IMG(packed, L.split_fwd[8]), 256, PB(packed, L, 8), w.XC, kColorPad, Q, 256, 0, st));       // feature
-    NSB_TRY(gemm_fwd(w.XC, kColorPad, PW(packed, L, 10), IMG(packed, L.split_fwd[10]), kColorPad, PB(packed, L, 10), w.C, kColorHidden, Q, 128, 1, st));  // color_fc
+    NSB_TRY(gemm_fwd(H8, kHidden, IMG(packed, L.split_fwd[8]), 256, PB(packed, L, 8), w.XC, kColorPad, Q, 256, 0, st));       // feature
+    NSB_TRY(gemm_fwd(w.XC, kColorPad, IMG(packed, L.split_fwd[10]), kColorPad, PB(packed, L, 10), w.C, kColorHidden, Q, 128, 1, st));  // color_fc
     head_fwd_kernel<<<elem_grid(Q * 32), 256, 0, st>>>(w.C, H8, kHidden, PW(packed, L, 11), PB(packed, L, 11),
                                                       PW(packed, L, 9), PB(packed, L, 9), raw, Q);
     NSB_LAUNCH_CHECK("head_fwd_kernel");
@@ -652,7 +477,7 @@ int fp32_mlp_fwd(const void* packed, float* raw, void* ws, int64_t Q, int stash,
 int fp32_mlp_bwd(const float* d_raw, const void* packed, float* grads, float* d_enc_pos, float* d_enc_dir, void* ws, int64_t Q,
                  cudaStream_t st) {
     const PackedLayout L = packed_layout();
-    Fp32Ws w = carve_fp32(ws, Q, 1);
+    Fp32Ws w = carve_fp32(ws, Q);
     const float* H8 = w.out[7];
     const LayerDesc dsg = layer_desc(9), dco = layer_desc(11), dfc = layer_desc(10), dft = layer_desc(8);
     auto G = [&](int64_t off) { return grads ? grads + off : nullptr; };
@@ -662,15 +487,14 @@ int fp32_mlp_bwd(const float* d_raw, const void* packed, float* grads, float* d_
                                              G(dco.w_off), G(dco.b_off), G(dsg.w_off), G(dsg.b_off), Q);
     NSB_LAUNCH_CHECK("head_bwd_kernel");
     if (d_enc_dir)
-        NSB_TRY(gemm_dinput(w.dC, kColorHidden, PW(packed, L, 10) + kHidden, IMG(packed, L.split_dinput[2]), kColorPad, d_enc_dir, kDirDim, Q,
-                            kColorHidden, 32, kDirDim, nullptr, st));
+        NSB_TRY(gemm_dinput(w.dC, kColorHidden, IMG(packed, L.split_dinput[2]), d_enc_dir, kDirDim, Q, kColorHidden, 32, kDirDim, nullptr, st));
     if (!grads && !d_enc_pos) return NSB_OK;
     // color_fc
     if (grads) NSB_TRY(gemm_wgrad(w.dC, kColorHidden, w.XC, kColorPad, grads + dfc.w_off, grads + dfc.b_off, Q, 128, dfc.K, dfc.Kpad, st));
-    NSB_TRY(gemm_dgrad(w.dC, kColorHidden, PW(packed, L, 10), IMG(packed, L.split_dgrad[10]), kColorPad, w.dB, kHidden, Q, 128, 256, nullptr, 0, nullptr, 0, st));  // dFeat
+    NSB_TRY(gemm_dgrad(w.dC, kColorHidden, IMG(packed, L.split_dgrad[10]), w.dB, kHidden, Q, 128, 256, nullptr, 0, nullptr, 0, st));  // dFeat
     // feature (no activation); dH8 = (dFeat.Wf + dsigma*w_sigma) * (H8>0)
     if (grads) NSB_TRY(gemm_wgrad(w.dB, kHidden, H8, kHidden, grads + dft.w_off, grads + dft.b_off, Q, 256, 256, 256, st));
-    NSB_TRY(gemm_dgrad(w.dB, kHidden, PW(packed, L, 8), IMG(packed, L.split_dgrad[8]), 256, w.dA, kHidden, Q, 256, 256, H8, kHidden, w.dA, kHidden, st));
+    NSB_TRY(gemm_dgrad(w.dB, kHidden, IMG(packed, L.split_dgrad[8]), w.dA, kHidden, Q, 256, 256, H8, kHidden, w.dA, kHidden, st));
     float* dcur = w.dA; float* dnext = w.dB;
     for (int l = 7; l >= 0; --l) {
         const LayerDesc d = layer_desc(l);
@@ -678,15 +502,13 @@ int fp32_mlp_bwd(const float* d_raw, const void* packed, float* grads, float* d_
         const int64_t ldx = l == 0 ? kPosPad : (l == 4 ? kSkipPad : w.out_ld[l - 1]);
         if (grads) NSB_TRY(gemm_wgrad(dcur, kHidden, Xin, ldx, grads + d.w_off, grads + d.b_off, Q, 256, d.K, d.Kpad, st));
         if (d_enc_pos && l == 4)        // the gamma(x) slab of the skip input, before the ping-pong overwrites dY_4
-            NSB_TRY(gemm_dinput(dcur, kHidden, PW(packed, L, 4) + kHidden, IMG(packed, L.split_dinput[1]), kSkipPad, d_enc_pos, kPosDim, Q,
-                                kHidden, kPosPad, kPosDim, nullptr, st));
+            NSB_TRY(gemm_dinput(dcur, kHidden, IMG(packed, L.split_dinput[1]), d_enc_pos, kPosDim, Q, kHidden, kPosPad, kPosDim, nullptr, st));
         if (d_enc_pos && l == 0)
-            NSB_TRY(gemm_dinput(dcur, kHidden, PW(packed, L, 0), IMG(packed, L.split_dinput[0]), kPosPad, d_enc_pos, kPosDim, Q, kHidden, kPosPad,
-                                kPosDim, d_enc_pos, st));
+            NSB_TRY(gemm_dinput(dcur, kHidden, IMG(packed, L.split_dinput[0]), d_enc_pos, kPosDim, Q, kHidden, kPosPad, kPosDim, d_enc_pos, st));
         if (l > 0) {
             // input of layer l is relu(out[l-1]) -> mask by out[l-1] > 0 (first 256 columns only at the skip layer)
-            NSB_TRY(gemm_dgrad(dcur, kHidden, PW(packed, L, l), IMG(packed, L.split_dgrad[l]), d.Kpad, dnext, kHidden, Q, 256, 256, w.out[l - 1],
-                               w.out_ld[l - 1], nullptr, 0, st));
+            NSB_TRY(gemm_dgrad(dcur, kHidden, IMG(packed, L.split_dgrad[l]), dnext, kHidden, Q, 256, 256, w.out[l - 1], w.out_ld[l - 1],
+                               nullptr, 0, st));
             float* t = dcur; dcur = dnext; dnext = t;
         }
     }

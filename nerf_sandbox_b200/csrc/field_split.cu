@@ -2,11 +2,10 @@
 //
 // The fp32 mode keeps every activation and gradient in HBM as fp32 (field_fp32.cu: concat-free buffers, one GEMM per layer
 // and role).  This file runs those GEMMs on tcgen05 without giving up fp32 accuracy: each fp32 operand element is split on
-// the fly into NT bf16 terms  x = x0 + x1 (+ x2)  (x0 = bf16(x), x1 = bf16(x - x0), ...; bf16 keeps fp32's exponent, so
+// the fly into three bf16 terms  x = x0 + x1 + x2  (x0 = bf16(x), x1 = bf16(x - x0), ...; bf16 keeps fp32's exponent, so
 // activations, weights and the tiny back-propagated gradients all split without scaling), and the product is the sum of the
-// term products with i + j < NT (3 MMAs for NT = 2, 6 for NT = 3), accumulated in fp32 in TMEM: x0 * y0 in one accumulator,
-// the cross products in a second one (see the MMA loop for why).  NT = 3 carries 24 significand bits per operand -- the same
-// information as the FFMA path.
+// six term products with i + j < 3, accumulated in fp32 in TMEM: x0 * y0 in one accumulator, the cross products in a second
+// one (see the MMA loop for why).  Three terms carry 24 significand bits per operand -- all of an fp32 operand.
 //
 // One CTA = one 128 x BN output tile (BN = 128 for forward / dgrad with two CTAs per SM, 256 for wgrad with one): 256
 // converter threads, an MMA warp and a producer warp.  Per K = 16 chunk every converter thread owns one 8-element piece of
@@ -17,11 +16,10 @@
 // MMA costs 3-4x more, DESIGN section 4).  The MMA warp issues the products of a chunk once all its pieces are written
 // (mbarrier) and commits them to the stage's "empty" barrier; the stage is rewritten only after that commit has arrived.
 // Forward and dgrad take B from term images of the weights written once per optimiser step (split_pack_kernel): the
-// producer warp bulk-copies them straight into the stage.  Epilogues as in field_fp32.cu -- bias + ReLU; addend + mask;
+// producer warp bulk-copies them straight into the stage.  Epilogues by role -- bias + ReLU; addend + mask;
 // split-K atomics, plus the bias gradient (column sums of wgrad's A pieces) -- staged through shared memory so that global
 // memory sees whole 512-byte rows.  What bounds it is shared-memory bandwidth (DESIGN section 2), not the tensor cores.
 #include <cuda_bf16.h>
-#include <cstdlib>
 #include "nsb_common.cuh"
 #include "tc_ptx.cuh"
 
@@ -37,20 +35,20 @@ constexpr int SG_THREADS = SG_CONV + 64;                              // + the M
 constexpr int SG_TERM_BYTES = SG_BM * SG_BK * 2;                      // one bf16 term image of a 128 x 16 operand chunk: [k/8][row][8]
 constexpr int SG_RAW_BYTES = SG_BM * SG_BK * 4;                       // the same chunk as fp32
 constexpr int SG_FIFO = 4;                                            // raw chunks in flight per CTA (cp.async groups)
-constexpr int SG_IMG_TERMS = 3;                                       // pre-split weight images always carry three terms
-constexpr int SG_IMG_CHUNK = SG_IMG_TERMS * SG_TERM_BYTES;            // 12 KB per (128-row tile, K = 16 chunk)
+constexpr int SG_TERMS = 3;                                           // bf16 terms per fp32 operand element (operands and weight images)
+constexpr int SG_IMG_CHUNK = SG_TERMS * SG_TERM_BYTES;                // 12 KB per (128-row tile, K = 16 chunk)
 // TMEM: two fp32 accumulators of BN columns: main (x0 * y0) and cross (every other term product)
 
-template <int NT, int BN> struct SgCfg {
+template <int BN> struct SgCfg {
     static constexpr int kBTiles = BN / 128;                              // B is handled as 128-row operand chunks
-    static constexpr int kStageBytes = (1 + kBTiles) * NT * SG_TERM_BYTES;   // converted stage: A terms, then B terms ([term][k/8][BN rows][8])
+    static constexpr int kStageBytes = (1 + kBTiles) * SG_TERMS * SG_TERM_BYTES;   // converted stage: A terms, then B terms ([term][k/8][BN rows][8])
     static constexpr int kStages = 2;
     static constexpr int kFifoOfs = kStages * kStageBytes;
     static constexpr int kFifoSlot = (1 + kBTiles) * SG_RAW_BYTES;        // raw chunk: A, then B
     static constexpr int kBarOfs = kFifoOfs + SG_FIFO * kFifoSlot;
     static constexpr int kEpiLd = BN + 4;                                 // row stride (floats) of the epilogue's shared-memory tile
     static_assert(kBarOfs >= SG_BM * kEpiLd * 4, "the epilogue tile reuses the stage + FIFO area");
-    static constexpr int kSmemBytes = kBarOfs + 128;                      // + barriers and the TMEM slot; NT = 3: 112.1 KB (BN 128) / 168.1 KB (BN 256)
+    static constexpr int kSmemBytes = kBarOfs + 128;                      // + barriers and the TMEM slot: 112.1 KB (BN 128) / 168.1 KB (BN 256)
     static constexpr uint32_t kTmemCols = 2 * BN;
 };
 
@@ -60,16 +58,15 @@ __device__ __forceinline__ uint32_t pack_bf16_pair(float lo, float hi) {
     return d;
 }
 
-// x[0..8) -> NT bf16 term vectors (16 bytes each); the residual of each step is exact in fp32
-template <int NT>
-__device__ __forceinline__ void split8(float (&x)[8], uint4 (&out)[NT]) {
+// x[0..8) -> SG_TERMS bf16 term vectors (16 bytes each); the residual of each step is exact in fp32
+__device__ __forceinline__ void split8(float (&x)[8], uint4 (&out)[SG_TERMS]) {
 #pragma unroll
-    for (int t = 0; t < NT; ++t) {
+    for (int t = 0; t < SG_TERMS; ++t) {
         uint32_t p[4];
 #pragma unroll
         for (int j = 0; j < 4; ++j) p[j] = pack_bf16_pair(x[2 * j], x[2 * j + 1]);
         out[t] = make_uint4(p[0], p[1], p[2], p[3]);
-        if (t + 1 < NT) {
+        if (t + 1 < SG_TERMS) {
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
                 x[2 * j] -= __uint_as_float(p[j] << 16);
@@ -119,7 +116,7 @@ __device__ __forceinline__ void sg_fetch(const float* __restrict__ P, int64_t ld
     }
 }
 // read this thread's slot back, split, write the term images of the converted stage
-template <bool TR, int NT, int ROWS = 128>       // ROWS: rows of the operand image this piece belongs to (k-group stride = 16 ROWS bytes)
+template <bool TR, int ROWS = 128>       // ROWS: rows of the operand image this piece belongs to (k-group stride = 16 ROWS bytes)
 __device__ __forceinline__ float sg_convert(const uint8_t* slot, uint8_t* img, int tid, int row_ofs = 0) {
     float x[8];
     if (!TR) {
@@ -132,19 +129,19 @@ __device__ __forceinline__ float sg_convert(const uint8_t* slot, uint8_t* img, i
     const float sum8 = ((x[0] + x[1]) + (x[2] + x[3])) + ((x[4] + x[5]) + (x[6] + x[7]));      // wgrad: this piece of the bias gradient
     int r, kg;
     sg_task<TR>(tid, r, kg);
-    uint4 terms[NT];
-    split8<NT>(x, terms);
+    uint4 terms[SG_TERMS];
+    split8(x, terms);
 #pragma unroll
-    for (int t = 0; t < NT; ++t) *reinterpret_cast<uint4*>(img + t * (ROWS * SG_BK * 2) + kg * (ROWS * 16) + (row_ofs + r) * 16) = terms[t];
+    for (int t = 0; t < SG_TERMS; ++t) *reinterpret_cast<uint4*>(img + t * (ROWS * SG_BK * 2) + kg * (ROWS * 16) + (row_ofs + r) * 16) = terms[t];
     return sum8;
 }
 
 // BIMG: the B operand is a weight matrix whose term images were written once per optimiser step (split_pack_kernel): a
 // producer thread bulk-copies the 4 KB term images of each chunk straight into the converted stage, and the converter
 // threads only handle A.
-template <bool AT, bool BT, int EPI, int NT, bool BIMG, int BN>
+template <bool AT, bool BT, int EPI, bool BIMG, int BN>
 __global__ void __launch_bounds__(SG_THREADS, BN == 128 ? 2 : 1) split_gemm_kernel(const GemmArgs g, int tiles_n, int tiles_mn) {
-    using Cfg = SgCfg<NT, BN>;
+    using Cfg = SgCfg<BN>;
     static_assert(BN == 128 || !BIMG, "weight images are tiled for 128 columns");
     extern __shared__ __align__(1024) uint8_t smem[];
     const uint32_t sbase = smem_u32(smem);
@@ -214,11 +211,11 @@ __global__ void __launch_bounds__(SG_THREADS, BN == 128 ? 2 : 1) split_gemm_kern
             if (use > 0) mbar_wait(bar_empty + 8 * s, (uint32_t)((use - 1) & 1));      // the MMAs that read this stage have completed
             const uint8_t* slot = smem + Cfg::kFifoOfs + (c % SG_FIFO) * Cfg::kFifoSlot;
             uint8_t* stage = smem + s * Cfg::kStageBytes;
-            colsum += sg_convert<AT, NT>(slot, stage, tid);
+            colsum += sg_convert<AT>(slot, stage, tid);
             if (!BIMG) {
 #pragma unroll
                 for (int h = 0; h < Cfg::kBTiles; ++h)
-                    sg_convert<BT, NT, BN>(slot + (1 + h) * SG_RAW_BYTES, stage + NT * SG_TERM_BYTES, tid, 128 * h);
+                    sg_convert<BT, BN>(slot + (1 + h) * SG_RAW_BYTES, stage + SG_TERMS * SG_TERM_BYTES, tid, 128 * h);
             }
             fence_async_smem();
             mbar_arrive(bar_full + 8 * s);
@@ -236,19 +233,19 @@ __global__ void __launch_bounds__(SG_THREADS, BN == 128 ? 2 : 1) split_gemm_kern
                 const int s = (int)(c % Cfg::kStages);
                 mbar_wait(bar_full + 8 * s, (uint32_t)((c / Cfg::kStages) & 1));
                 tc_fence_after();
-                const uint32_t a0 = sbase + s * Cfg::kStageBytes, b0 = a0 + NT * SG_TERM_BYTES;
+                const uint32_t a0 = sbase + s * Cfg::kStageBytes, b0 = a0 + SG_TERMS * SG_TERM_BYTES;
                 // Two accumulators.  tcgen05 adds each MMA into the fp32 accumulator with TRUNCATION (measured: same-sign sums
                 // come out low by ~0.25 ulp per MMA, scripts/dbg_split_gemm.py), so the error grows with the number of MMAs that
                 // touch an accumulator of full magnitude.  Only the x0 * y0 product (K / 16 MMAs) goes to the main accumulator;
-                // the 2 (NT = 2) or 5 (NT = 3) cross products are 2^-8 .. 2^-16 of it and collect in their own accumulator,
+                // the 5 cross products are 2^-8 .. 2^-16 of it and collect in their own accumulator,
                 // where their truncation is that much smaller; the epilogue adds the two in registers (round to nearest).
 #pragma unroll
-                for (int sum = NT - 1; sum >= 1; --sum) {          // smallest products first
+                for (int sum = SG_TERMS - 1; sum >= 1; --sum) {          // smallest products first
 #pragma unroll
                     for (int ta = 0; ta <= sum; ++ta) {
                         const int tb = sum - ta;
                         tc_mma(tmem_base + BN, desc_at(dhi, a0 + ta * SG_TERM_BYTES), desc_at(dhi_b, b0 + tb * kBTerm), idesc,
-                               (c == 0 && sum == NT - 1 && ta == 0) ? 0u : 1u);
+                               (c == 0 && sum == SG_TERMS - 1 && ta == 0) ? 0u : 1u);
                     }
                 }
                 tc_mma(tmem_base, desc_at(dhi, a0), desc_at(dhi_b, b0), idesc, c == 0 ? 0u : 1u);
@@ -257,14 +254,14 @@ __global__ void __launch_bounds__(SG_THREADS, BN == 128 ? 2 : 1) split_gemm_kern
             }
         }
     } else if (BIMG && lane == 0) {
-        // ---- weight-image producer: chunk c of column tile tn = NT contiguous 4 KB term images
+        // ---- weight-image producer: chunk c of column tile tn = SG_TERMS contiguous 4 KB term images
         const uint8_t* img = g.b_img + ((size_t)tn * (size_t)(g.Kdim / SG_BK) + (size_t)(kbeg / SG_BK)) * SG_IMG_CHUNK;
         for (int64_t c = 0; c < nchunks; ++c) {
             const int s = (int)(c % Cfg::kStages);
             const int64_t use = c / Cfg::kStages;
             if (use > 0) mbar_wait(bar_empty + 8 * s, (uint32_t)((use - 1) & 1));
-            mbar_expect_tx(bar_full + 8 * s, NT * SG_TERM_BYTES);
-            bulk_g2s(sbase + s * Cfg::kStageBytes + NT * SG_TERM_BYTES, img + (size_t)c * SG_IMG_CHUNK, NT * SG_TERM_BYTES, bar_full + 8 * s);
+            mbar_expect_tx(bar_full + 8 * s, SG_IMG_CHUNK);
+            bulk_g2s(sbase + s * Cfg::kStageBytes + SG_TERMS * SG_TERM_BYTES, img + (size_t)c * SG_IMG_CHUNK, SG_IMG_CHUNK, bar_full + 8 * s);
         }
     }
     cp_async_wait<0>();
@@ -370,18 +367,18 @@ __global__ void __launch_bounds__(256) split_pack_kernel(const float* __restrict
             const int k = k0 + j;
             x[j] = (n < jb.n_true && k < jb.k_true) ? params[jb.w_off + (jb.transpose ? (int64_t)k * jb.ldw + n : (int64_t)n * jb.ldw + k)] : 0.f;
         }
-        uint4 terms[SG_IMG_TERMS];
-        split8<SG_IMG_TERMS>(x, terms);
+        uint4 terms[SG_TERMS];
+        split8(x, terms);
         uint8_t* dst = base + jb.dst + (size_t)tc_ * SG_IMG_CHUNK + kg * 2048 + r * 16;
 #pragma unroll
-        for (int t = 0; t < SG_IMG_TERMS; ++t) *reinterpret_cast<uint4*>(dst + t * SG_TERM_BYTES) = terms[t];
+        for (int t = 0; t < SG_TERMS; ++t) *reinterpret_cast<uint4*>(dst + t * SG_TERM_BYTES) = terms[t];
     }
 }
 
-template <bool AT, bool BT, int EPI, int NT, bool BIMG, int BN = 128>
+template <bool AT, bool BT, int EPI, bool BIMG, int BN = 128>
 static int launch_split_gemm(const GemmArgs& g, cudaStream_t st) {
-    using Cfg = SgCfg<NT, BN>;
-    auto kern = split_gemm_kernel<AT, BT, EPI, NT, BIMG, BN>;
+    using Cfg = SgCfg<BN>;
+    auto kern = split_gemm_kernel<AT, BT, EPI, BIMG, BN>;
     static bool configured = false;          // per instantiation
     if (!configured) {
         if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes) != cudaSuccess)
@@ -410,12 +407,6 @@ static int launch_split_gemm(const GemmArgs& g, cudaStream_t st) {
 
 }  // namespace tc
 
-// number of bf16 terms per operand: NSB_SPLIT_TERMS=2 -> 16 significand bits (3 MMAs), default 3 -> 24 bits (6 MMAs)
-static int split_terms() {
-    static const int nt = [] { const char* e = getenv("NSB_SPLIT_TERMS"); return (e && e[0] == '2') ? 2 : 3; }();
-    return nt;
-}
-
 size_t split_image_bytes(int n_rows, int k_len) { return (size_t)cdiv(n_rows, 128) * (size_t)(k_len / 16) * tc::SG_IMG_CHUNK; }
 
 // Every weight image of a net: forward B = W (n = out feature, k = in feature, zero beyond K), dgrad B = W^T restricted to
@@ -442,42 +433,33 @@ int split_pack(const float* params, void* packed, cudaStream_t st) {
     return NSB_OK;
 }
 
-// NSB_SPLIT_WGRAD_WIDE=0: 128-column CTAs for wgrad too (A/B timing)
-static bool wgrad_wide() {
-    static const bool w = [] { const char* e = getenv("NSB_SPLIT_WGRAD_WIDE"); return !(e && e[0] == '0'); }();
-    return w;
-}
-
 int split_gemm(const GemmArgs& g, int role, cudaStream_t st) {
     NSB_TRY(check_arch());
     // alignment contract of the loaders / epilogues (all layer buffers of field_fp32.cu satisfy it)
     const bool any_ldc = role == EPI_DGRAD && g.n_valid > 0;        // input gradients: scalar epilogue, any row stride
     if ((g.lda & 3) || (g.ldb & 3) || (role != EPI_WGRAD && ((g.Kdim & 15) || ((g.ldc & 3) && !any_ldc) || (g.Ndim & 15)))) return NSB_E_BADARG;
-    const bool t3 = split_terms() == 3;
     const bool img = g.b_img != nullptr && role != EPI_WGRAD;
-#define NSB_SG(AT, BT, EPI, IMGF) (t3 ? tc::launch_split_gemm<AT, BT, EPI, 3, IMGF>(g, st) : tc::launch_split_gemm<AT, BT, EPI, 2, IMGF>(g, st))
     switch (role) {
-        case EPI_FWD: return img ? NSB_SG(false, false, EPI_FWD, true) : NSB_SG(false, false, EPI_FWD, false);
-        case EPI_DGRAD: return img ? NSB_SG(false, true, EPI_DGRAD, true) : NSB_SG(false, true, EPI_DGRAD, false);
+        case EPI_FWD: return img ? tc::launch_split_gemm<false, false, EPI_FWD, true>(g, st) : tc::launch_split_gemm<false, false, EPI_FWD, false>(g, st);
+        case EPI_DGRAD: return img ? tc::launch_split_gemm<false, true, EPI_DGRAD, true>(g, st) : tc::launch_split_gemm<false, true, EPI_DGRAD, false>(g, st);
         case EPI_WGRAD: {
             // 256-column CTAs over the whole multiples of 256 columns of B, 128-column CTAs over the rest (gamma(x) / gamma(d)
             // columns of the skip and colour layers, layer 0); the bias gradient rides with the first launch only
-            const int64_t wide = wgrad_wide() ? g.Ndim / 256 * 256 : 0;
+            const int64_t wide = g.Ndim / 256 * 256;
             if (wide > 0) {
                 GemmArgs a = g;
                 a.Ndim = wide; a.n_valid = g.n_valid < wide ? g.n_valid : (int)wide;
-                NSB_TRY(t3 ? (tc::launch_split_gemm<true, true, EPI_WGRAD, 3, false, 256>(a, st)) : (tc::launch_split_gemm<true, true, EPI_WGRAD, 2, false, 256>(a, st)));
+                NSB_TRY((tc::launch_split_gemm<true, true, EPI_WGRAD, false, 256>(a, st)));
             }
             if (wide < g.Ndim) {
                 GemmArgs a = g;
                 a.B = g.B + wide; a.C = g.C + wide; a.Ndim = g.Ndim - wide; a.n_valid = g.n_valid - (int)wide;
                 if (wide > 0) a.colsum = nullptr;
-                if (a.n_valid > 0) return t3 ? (tc::launch_split_gemm<true, true, EPI_WGRAD, 3, false, 128>(a, st)) : (tc::launch_split_gemm<true, true, EPI_WGRAD, 2, false, 128>(a, st));
+                if (a.n_valid > 0) return tc::launch_split_gemm<true, true, EPI_WGRAD, false, 128>(a, st);
             }
             return NSB_OK;
         }
     }
-#undef NSB_SG
     return NSB_E_BADARG;
 }
 

@@ -44,10 +44,6 @@ constexpr int kSmemBias = kSmemBar + 256;                   // 2 x 1 KB: per epi
 constexpr int kSmemBytes = kSmemBias + 2048;
 constexpr int kThreads = 384;
 // forward kernel, CTA pair: a ring stage holds this CTA's half of a K=32 slab (N/2 weight rows) -> twice the stages
-#ifndef NSB_SHARE_SLABS
-#define NSB_SHARE_SLABS 1
-#endif
-constexpr bool kShareSlabs = NSB_SHARE_SLABS != 0;
 constexpr int kStages2 = 8;
 constexpr int kStageBytes2 = kStageBytes / 2;
 static_assert(8 * (3 * kStages2 + 6) + 4 <= 256, "barrier block overflow");
@@ -111,25 +107,14 @@ __device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
     return *reinterpret_cast<uint32_t*>(&t);
 }
 // fp16 pair {lo = a, hi = b}, saturating at +-65504 instead of overflowing to inf; _relu clamps negatives to +0 first
-#ifndef NSB_F16_SAT
-#define NSB_F16_SAT 1
-#endif
 __device__ __forceinline__ uint32_t pack_f16(float a, float b) {
     uint32_t d;
-#if NSB_F16_SAT
     asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(b), "f"(a));
-#else
-    asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(b), "f"(a));
-#endif
     return d;
 }
 __device__ __forceinline__ uint32_t pack_f16_relu(float a, float b) {
     uint32_t d;
-#if NSB_F16_SAT
     asm("cvt.rn.relu.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(b), "f"(a));
-#else
-    asm("cvt.rn.relu.f16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(b), "f"(a));
-#endif
     return d;
 }
 template <bool F16> __device__ __forceinline__ uint32_t pack2(float a, float b) { return F16 ? pack_f16(a, b) : pack_bf16(a, b); }
@@ -428,7 +413,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) field_f
                     const int ns = layer_nslabs(l);
                     // a layer whose slabs fit the ring is fetched once and used by tile A, then by tile B; the two longer
                     // layers (the skip layer and color_fc) are streamed once per tile
-                    for (int s2 = 0; s2 < (kShareSlabs && ns <= kStages2 ? ns : 2 * ns); ++s2) {
+                    for (int s2 = 0; s2 < (ns <= kStages2 ? ns : 2 * ns); ++s2) {
                         const int s = s2 >= ns ? s2 - ns : s2;
                         mbar_wait_t(bar_empty + 8 * stage, (round & 1) ^ 1, w_empty);
                         if (elect_one()) {
@@ -485,7 +470,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) field_f
                     // A-operand segments of the layer: n_act slabs from the activation buffer, then n_gx from the gamma buffer
                     const int n_act = l == 0 ? 0 : 8;
                     const int n_gx = l == 0 ? 2 : (l == 4 ? 2 : (l == 9 ? 1 : 0));
-                    const bool shared = kShareSlabs && n_act + n_gx <= kStages2;       // slabs fetched once, used by tile A then tile B
+                    const bool shared = n_act + n_gx <= kStages2;       // slabs fetched once, used by tile A then tile B
                     const uint32_t stage0 = stage, round0 = round;
                     for (int t = 0; t < 2; ++t) {
                         if (p.cyc) mbar_wait_t(bar_in + 8 * t, use & 1, w_in); else mbar_wait(bar_in + 8 * t, use & 1);
@@ -1291,7 +1276,7 @@ struct WgradJob {
 constexpr int kMaxJobs = 16;
 struct WgradParams {
     const uint8_t* stash; const uint8_t* dstash; const float* d_raw; float* grads;
-    int64_t num_tiles, Q; int num_jobs; int dbg; int rev;
+    int64_t num_tiles, Q; int num_jobs; int dbg;
     WgradJob jobs[kMaxJobs];
 };
 constexpr int kWgPiece = 32768;                       // ring slot: one column half of a tile image
@@ -1371,7 +1356,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) field_wgrad_kernel(const __grid
                 const WgPiece& pc = job.pieces[i];
                 // tiles are walked from the LAST one down: dgrad has just written the gradient stash front to back, so its tail (as much
                 // as the 126 MB L2 still holds) is read back without going to HBM
-                const int64_t pt = p.rev ? p.num_tiles - 1 - tile : tile;
+                const int64_t pt = p.num_tiles - 1 - tile;
                 const uint8_t* src = pc.from_stash ? p.stash + (size_t)pt * kStashTile + pc.ofs : p.dstash + (size_t)pt * kDstashTile + pc.ofs;
                 mbar_wait(bar_empty + 8 * slot, (round & 1) ^ 1);
                 if (elect_one()) {
@@ -1434,7 +1419,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) field_wgrad_kernel(const __grid
         auto load_dr = [&](int64_t tile, float4 (&dr)[4]) {
 #pragma unroll
             for (int rg = 0; rg < 4; ++rg) {
-                const int64_t q = (p.rev ? p.num_tiles - 1 - tile : tile) * TILE_M + rg * 32 + lane;
+                const int64_t q = (p.num_tiles - 1 - tile) * TILE_M + rg * 32 + lane;
                 dr[rg] = (tile < p.num_tiles && q < p.Q) ? __ldg(reinterpret_cast<const float4*>(p.d_raw) + q) : make_float4(0.f, 0.f, 0.f, 0.f);
             }
         };
@@ -1985,7 +1970,6 @@ int tc_field_bwd(const float* d_raw, const void* packed, float* grads, float* d_
     }
     wp.num_jobs = nj;
     wp.dbg = getenv("NSB_WG_DBG") != nullptr;
-    { static const int rev = [] { const char* e = getenv("NSB_WG_REVERSE"); return (e && e[0] == '0') ? 0 : 1; }(); wp.rev = rev; }
     // CTAs per job: greedy min-max of (tiles per CTA) x (cycles per tile).  The per-tile cost is what the MMA thread of
     // each job kind was measured to take on B200 (scripts/perf_bwd.py with NSB_WG_DBG=1): an MN-major MMA costs
     // ~200-250 cycles whatever its N, so cost follows the instruction count more than the bytes.

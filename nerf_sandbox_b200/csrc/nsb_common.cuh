@@ -146,8 +146,8 @@ __host__ __device__ inline LayerDesc layer_desc(int l) {
     return d;
 }
 
-// One layer GEMM of the fp32 mode, C[m,n] = sum_k A(m,k) * B(n,k), with the epilogue of its role (field_fp32.cu: FFMA
-// tiles; field_split.cu: the same contract on the tensor cores with bf16-split operands).
+// One layer GEMM of the fp32 mode, C[m,n] = sum_k A(m,k) * B(n,k), with the epilogue of its role (field_split.cu: on the
+// tensor cores with bf16-split operands).
 // AT = false: A stored [m][k] (k contiguous), AT = true: A stored [k][m]; same for BT and B.
 enum { EPI_FWD = 0, EPI_DGRAD = 1, EPI_WGRAD = 2 };
 struct GemmArgs {
@@ -161,8 +161,8 @@ struct GemmArgs {
     int n_valid;                        // WGRAD: columns < n_valid are written; DGRAD: when > 0, only columns < n_valid are
                                         //   written (and addend read), with scalar accesses: C / addend of any leading dimension
     int64_t k_per_split;                // WGRAD: contraction rows per split
-    float* colsum;                      // WGRAD on the tensor cores: += column sums of A (the bias gradient), or null
-    const uint8_t* b_img;               // FWD / DGRAD on the tensor cores: pre-split term images of B (split_pack), or null
+    float* colsum;                      // WGRAD: += column sums of A (the bias gradient), or null
+    const uint8_t* b_img;               // FWD / DGRAD: pre-split term images of B (split_pack), or null
 };
 // field_split.cu: role = EPI_* (FWD: A, B k-contiguous; DGRAD: B stored [k][n]; WGRAD: both stored [k][.], split-K with atomics)
 int split_gemm(const GemmArgs& g, int role, cudaStream_t st);

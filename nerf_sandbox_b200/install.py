@@ -131,7 +131,7 @@ def _fused_train_step(original):
 def install(verbose: bool = False, mode: str | None = None, fuse_train_step: bool = True) -> dict:
     """Rebind the reference's names; returns {module: [names rebound]}.  The reference package must be importable.
 
-    ``mode`` ("bf16" = tcgen05 tensor cores, "fp32" = FFMA parity kernels; default: NSB_MODE, else "fp32") becomes the
+    ``mode`` ("bf16" = bf16 tensor-core kernels, "fp32" = parity kernels; default: NSB_MODE, else "fp32") becomes the
     arithmetic mode of every ``NeRF`` the reference builds afterwards -- its Trainer passes no mode (train/trainer.py:326-341),
     so this is how ``train_nerf.py --vanilla`` reaches the tensor-core path.
 

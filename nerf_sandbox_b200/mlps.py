@@ -1,5 +1,5 @@
 """NeRF MLP with the reference's module interface (models/mlps.py:35-314); forward and backward run in
-libnsb (fp32 FFMA mode or bf16 tcgen05 mode).  Parameters live in nn.Linear modules so ``state_dict``
+libnsb (fp32 parity mode or bf16 mode, both on tcgen05).  Parameters live in nn.Linear modules so ``state_dict``
 keeps the reference's keys/shapes (SURVEY section 5), but their storage is one flat fp32 buffer in
 state_dict order: the kernels, the gradient all-reduce and the fused Adam step all see a single array."""
 from __future__ import annotations
@@ -31,7 +31,7 @@ def log_nerf_arch(nerf, pos_enc=None, dir_enc=None, logger=print, name="NeRF"):
 
 # Arithmetic mode of NeRF modules built without an explicit ``mode=`` -- which is how the reference's Trainer builds them
 # (train/trainer.py:326-341 passes no such argument).  install(mode=...) / set_default_mode() / NSB_MODE select it:
-# "bf16" = tcgen05 tensor-core kernels, "fp32" = FFMA parity kernels.
+# "bf16" = bf16 tensor-core kernels, "fp32" = parity kernels (fp32 activations, split-operand tensor-core GEMMs).
 import os as _os
 _DEFAULT_MODE = _os.environ.get("NSB_MODE", "fp32").lower()
 
@@ -102,7 +102,7 @@ class _FieldEncFn(torch.autograd.Function):
 
 class NeRF(nn.Module):
     """8x256 trunk with the skip concat at the input of layer ``skip_pos``, raw [r,g,b,sigma] output
-    (models/mlps.py:41-134, :192-278).  ``mode``: "fp32" (FFMA, parity) or "bf16" (tcgen05); None = the package default
+    (models/mlps.py:41-134, :192-278).  ``mode``: "fp32" (parity) or "bf16"; None = the package default
     (set_default_mode / install(mode=...) / NSB_MODE), so the reference's own constructor call selects it."""
 
     def __init__(self, enc_pos_dim: int, enc_dir_dim: int, n_layers: int = 8, hidden_dim: int = 256, skip_pos: int = 4,

@@ -37,7 +37,8 @@ def _composite_ref(raw, z, rn, noise, flags_white=True, inf_last=True):
 
 @pytest.mark.parametrize("N", [1, 31, 37, 64, 100, 192, 255, 256, 257, 300])
 def test_raw_compositor_ragged_sizes_with_guards(N):
-    """N <= 256 runs the run-layout kernels (partial runs when N is not a multiple of 32), N > 256 the strided ones."""
+    """N <= 192 runs the one-warp run-layout kernels, 193..300 the multi-warp ones (partial runs when N is not a multiple of 32);
+    the strided kernels (N > 1024) are covered by test_gpu_parity.py::test_compositor_ragged_and_long_rays."""
     from nerf_sandbox_b200 import _lib
     L = _lib.lib(); st = _lib.stream()
     B = 37
@@ -105,9 +106,9 @@ def test_resample_merge_shapes_with_guards(nc, nf):
                 assert float(ok.float().mean()) > 0.99              # (index flips at CDF ties with u = 1.0 aside)
 
 
-def test_split_forward_ragged_sizes_matches_ffma_forward():
-    """fp32 mode: the no-grad forward (fp16-split tensor-core kernel) against the grad-enabled forward (FFMA kernels) on ragged
-    point counts, raw outputs within 1e-4 relative + 2e-5 absolute; guard zones around the output."""
+def test_split_forward_ragged_sizes_matches_training_forward():
+    """fp32 mode: the no-grad forward (fp16-split tensor-core kernel) against the grad-enabled forward (bf16-split layer GEMMs)
+    on ragged point counts, raw outputs within 1e-4 relative + 2e-5 absolute."""
     import nerf_sandbox_b200 as nsb
     from oracle import nerf_oracle as O
     net = nsb.NeRF(63, 27, mode="fp32").to(DEV)
