@@ -15,9 +15,9 @@
  *     the Python wrappers raise RuntimeError/ValueError like the reference does;
  *   - nullable arguments are marked [opt];
  *   - threading: the library keeps no state per call except (a) thread-local markers set for the duration of nsb_train_step
- *     and (b) ONE helper stream + event pair per device, created on first use, on which nsb_train_fwd_bwd / nsb_train_step
+ *     and (b) ONE helper stream + event pair per device, created on first use, on which nsb_train_fwd_bwd(_ex) / nsb_train_step
  *     run half batches and the coarse backward chain.  Calls on different devices are independent; on one device, two host
- *     threads must not be inside nsb_train_fwd_bwd / nsb_train_step at the same time (the reference is single-threaded,
+ *     threads must not be inside nsb_train_fwd_bwd(_ex) / nsb_train_step at the same time (the reference is single-threaded,
  *     single-stream; NSB_SIDE_STREAM=0 removes the helper stream and with it this restriction).
  */
 #ifndef NSB_H_
@@ -275,6 +275,26 @@ int nsb_train_fwd_bwd(const float* rays_o, const float* rays_d, const float* ray
                       int det_fine, int mode, float grad_scale, uint64_t seed, uint64_t step, const float* U,
                       const float* u_fine, const float* noise_c, const float* noise_f, void* stream);
 
+/* Workspace of nsb_train_fwd_bwd_ex: with ray_grads != 0 it holds the encoding gradients of both passes as well, 360 B more per
+ * point (B * (2 Nc + Nf) points).  ray_grads == 0 is nsb_train_workspace_bytes. */
+size_t nsb_train_workspace_bytes_ex(int64_t B, int Nc, int Nf, int mode, int ray_grads);
+
+/* nsb_train_fwd_bwd that also returns the gradient of the step's loss (times grad_scale) w.r.t. its rays -- what autograd gives
+ * rays_o, rays_d and viewdirs in the reference's _train_step: d_rays_o[B,3], d_rays_d[B,3], d_viewdirs[B,3], each [opt] and
+ * overwritten, each the sum of the coarse and the fine pass (fine first, then coarse, in a fixed order: bitwise repeatable).
+ * d_viewdirs needs viewdirs; without viewdirs the view-direction term goes to d_rays_d.  grads_c / grads_f: both or neither;
+ * neither (with a ray output) is a frozen field, and no weight-gradient kernel runs.  z and ray_norm get no gradient, so for
+ * NDC rays, whose marching norm depends on the pose, a pose gradient built on these is incomplete.  Workspace:
+ * nsb_train_workspace_bytes_ex(..., ray_grads = 1) when a ray output is given.  With no ray output this is nsb_train_fwd_bwd:
+ * the same launches in the same order. */
+int nsb_train_fwd_bwd_ex(const float* rays_o, const float* rays_d, const float* ray_norm, const float* viewdirs,
+                         const float* target, const void* packed_c, const void* packed_f, float* grads_c,
+                         float* grads_f, float* scalars, float* comp_c, float* comp_f, void* ws, size_t ws_bytes,
+                         int64_t B, int Nc, int Nf, float near_, float far_, float noise_std, uint32_t flags,
+                         int det_fine, int mode, float grad_scale, uint64_t seed, uint64_t step, const float* U,
+                         const float* u_fine, const float* noise_c, const float* noise_f, float* d_rays_o,
+                         float* d_rays_d, float* d_viewdirs, void* stream);
+
 size_t nsb_render_workspace_bytes(int64_t B, int Nc, int Nf, int mode);
 
 /* One ray tile of render_image_chunked, utils/render_utils.py:337-417 (perturb=False): coarse linspace,
@@ -299,6 +319,21 @@ int nsb_camera_rays(int H, int W, const float* K_host, const float* c2w_host, in
                     int pixel_center, int as_ndc, float near_plane, const float* pixels_xy, int64_t n_pixels,
                     float* o_world, float* d_world_unit, float* d_world_norm, float* o_march, float* d_march_unit,
                     float* d_march_norm, void* stream);
+
+/* Backward of nsb_camera_rays / nsb_sample_pixel_batch w.r.t. the poses (iNeRF / BARF-style pose refinement): the exact adjoint
+ * of the six outputs in world and NDC mode.  Ks[F,4] = (fx,fy,cx,cy) and c2ws[F,12] (row-major 3x4) are DEVICE arrays, as for
+ * the sampler; fids[n] [opt] is each ray's frame (NULL: every ray is frame 0; an id outside [0,F) contributes nothing) and
+ * pixels_xy[n,2] [opt] its pixel (NULL: the full row-major H*W grid, and then n must be H*W) -- what the sampler returns.
+ * Upstream gradients g_*[n,3] / g_*_norm[n], each [opt] (a missing one counts as zero), at least one given.
+ * d_c2ws[F,12] is overwritten with dL/dc2w[:3,:4]; a frame no ray belongs to gets exactly zero.  The per-frame sums use no
+ * atomics (block partials in ws, then a second pass in block order): bitwise repeatable.  ws: at least
+ * nsb_camera_rays_bwd_workspace_bytes(n, F) bytes.  Two launches. */
+size_t nsb_camera_rays_bwd_workspace_bytes(int64_t n, int F);
+int nsb_camera_rays_bwd(int H, int W, const float* Ks, const float* c2ws, int F, const int* fids, int convention,
+                        int pixel_center, int as_ndc, float near_plane, const float* pixels_xy, int64_t n,
+                        const float* g_o_world, const float* g_d_world_unit, const float* g_d_world_norm,
+                        const float* g_o_march, const float* g_d_march_unit, const float* g_d_march_norm,
+                        float* d_c2ws, void* ws, size_t ws_bytes, void* stream);
 
 /* Device-side pixel/ray batch sampler (SURVEY section 8f rank 2): RandomPixelRaySampler.__iter__,
  * data/samplers.py:134-290, with the images resident in HBM and no host round trip.  images[F,H,W,C] (C = 3 or 4,

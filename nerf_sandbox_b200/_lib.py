@@ -59,10 +59,15 @@ SIGNATURES = {
                                  _p, _p, _p, _p, _p]),
     "nsb_train_step": (_i32, [_p] * 14 + [_sz, _i64, _i32, _i32, _f32, _f32, _f32, _u32, _i32, _i32, _u64, _f32, _f32, _i64, _f32, _f32, _f32,
                               _f32, _p, _p, _p, _p, _p, _p, _p, _i32, _i32, _p]),
+    "nsb_train_workspace_bytes_ex": (_sz, [_i64, _i32, _i32, _i32, _i32]),
+    "nsb_train_fwd_bwd_ex": (_i32, [_p] * 13 + [_sz, _i64, _i32, _i32, _f32, _f32, _f32, _u32, _i32, _i32, _f32, _u64, _u64]
+                             + [_p] * 8),
     "nsb_render_workspace_bytes": (_sz, [_i64, _i32, _i32, _i32]),
     "nsb_render_rays": (_i32, [_p] * 10 + [_sz, _i64, _i32, _i32, _f32, _f32, _u32, _i32, _p]),
     "nsb_frame_output": (_i32, [_p, _p, _p, _i64, C.c_double, C.c_double, _i32, _p, _p, _p, _p, _p, _p, _p, _p]),
     "nsb_camera_rays": (_i32, [_i32, _i32, _p, _p, _i32, _i32, _i32, _i32, _f32, _p, _i64] + [_p] * 7),
+    "nsb_camera_rays_bwd_workspace_bytes": (_sz, [_i64, _i32]),
+    "nsb_camera_rays_bwd": (_i32, [_i32, _i32, _p, _p, _i32, _p, _i32, _i32, _i32, _f32, _p, _i64] + [_p] * 8 + [_sz, _p]),
     "nsb_sample_pixel_batch": (_i32, [_p, _i32, _i32, _i32, _i32, _p, _p, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _f32,
                                       _i64, _u64, _u64] + [_p] * 10),
 }

@@ -193,8 +193,11 @@ struct TrainWs {
     float *zc, *w_c, *z_all, *raw_c, *raw_f, *d_raw, *d_raw_c, *comp_c, *comp_f, *g_c, *g_f;
     void *field_c, *field_f;
     size_t field_c_bytes, field_f_bytes, bytes;
+    // ray gradients only (after everything above, so the layout without them is unchanged): encoding gradients of both passes
+    // (63 + 27 floats per point each: 360 B per point in all) and the coarse pass's d rays_o / rays_d / viewdirs [3][B,3]
+    float *d_ep_c, *d_ed_c, *d_ep_f, *d_ed_f, *d_rays_c;
 };
-TrainWs carve_train(void* base, int64_t B, int Nc, int Nf, int mode) {
+TrainWs carve_train(void* base, int64_t B, int Nc, int Nf, int mode, bool ray_grads) {
     TrainWs t;
     char* p = reinterpret_cast<char*>(base);
     size_t off = 0;
@@ -205,24 +208,46 @@ TrainWs carve_train(void* base, int64_t B, int Nc, int Nf, int mode) {
     t.comp_c = (float*)take(B * 12); t.comp_f = (float*)take(B * 12); t.g_c = (float*)take(B * 12); t.g_f = (float*)take(B * 12);
     t.field_c_bytes = field_ws(Qc, mode, 1); t.field_f_bytes = field_ws(Qf, mode, 1);
     t.field_c = take(t.field_c_bytes); t.field_f = take(t.field_f_bytes);
+    t.d_ep_c = t.d_ed_c = t.d_ep_f = t.d_ed_f = t.d_rays_c = nullptr;
+    if (ray_grads) {
+        t.d_ep_c = (float*)take(Qc * 63 * 4); t.d_ed_c = (float*)take(Qc * 27 * 4);
+        t.d_ep_f = (float*)take(Qf * 63 * 4); t.d_ed_f = (float*)take(Qf * 27 * 4);
+        t.d_rays_c = (float*)take(B * 36);
+    }
     t.bytes = off;
     return t;
+}
+// fine-pass ray gradients += the coarse pass's, in that order (after the join of the two backward chains)
+__global__ void add_coarse_ray_grads_kernel(float* __restrict__ d_o, float* __restrict__ d_d, float* __restrict__ d_v,
+                                            const float* __restrict__ coarse, int64_t n3) {
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n3; i += (int64_t)gridDim.x * blockDim.x) {
+        if (d_o) d_o[i] += coarse[i];
+        if (d_d) d_d[i] += coarse[n3 + i];
+        if (d_v) d_v[i] += coarse[2 * n3 + i];
+    }
 }
 }  // namespace
 
 extern "C" size_t nsb_train_workspace_bytes(int64_t B, int Nc, int Nf, int mode) {
-    return carve_train(nullptr, B, Nc, Nf, mode).bytes;
+    return carve_train(nullptr, B, Nc, Nf, mode, false).bytes;
+}
+extern "C" size_t nsb_train_workspace_bytes_ex(int64_t B, int Nc, int Nf, int mode, int ray_grads) {
+    return carve_train(nullptr, B, Nc, Nf, mode, ray_grads != 0).bytes;
 }
 
-extern "C" int nsb_train_fwd_bwd(const float* rays_o, const float* rays_d, const float* ray_norm, const float* viewdirs,
-                                 const float* target, const void* packed_c, const void* packed_f, float* grads_c,
-                                 float* grads_f, float* scalars, float* comp_c, float* comp_f, void* ws, size_t ws_bytes,
-                                 int64_t B, int Nc, int Nf, float near_, float far_, float noise_std, uint32_t flags,
-                                 int det_fine, int mode, float grad_scale, uint64_t seed, uint64_t step, const float* U,
-                                 const float* u_fine, const float* noise_c, const float* noise_f, void* stream) {
-    if (!rays_o || !rays_d || !target || !packed_c || !packed_f || !grads_c || !grads_f || !scalars || !ws) return NSB_E_BADARG;
+extern "C" int nsb_train_fwd_bwd_ex(const float* rays_o, const float* rays_d, const float* ray_norm, const float* viewdirs,
+                                    const float* target, const void* packed_c, const void* packed_f, float* grads_c,
+                                    float* grads_f, float* scalars, float* comp_c, float* comp_f, void* ws, size_t ws_bytes,
+                                    int64_t B, int Nc, int Nf, float near_, float far_, float noise_std, uint32_t flags,
+                                    int det_fine, int mode, float grad_scale, uint64_t seed, uint64_t step, const float* U,
+                                    const float* u_fine, const float* noise_c, const float* noise_f, float* d_rays_o,
+                                    float* d_rays_d, float* d_viewdirs, void* stream) {
+    const bool ray_grads = d_rays_o || d_rays_d || d_viewdirs;
+    if (!rays_o || !rays_d || !target || !packed_c || !packed_f || !scalars || !ws) return NSB_E_BADARG;
+    // both gradient buffers, or neither (a frozen field: then only the ray gradients are computed)
+    if (!grads_c != !grads_f || (!grads_c && !ray_grads) || (d_viewdirs && !viewdirs)) return NSB_E_BADARG;
     if (B < 1 || Nc < 2 || Nf < 1) return NSB_E_BADARG;
-    TrainWs t = carve_train(ws, B, Nc, Nf, mode);
+    TrainWs t = carve_train(ws, B, Nc, Nf, mode, ray_grads);
     if (ws_bytes < t.bytes) return NSB_E_WORKSPACE;
     cudaStream_t st = as_stream(stream);
     const int Nt = Nc + Nf;
@@ -230,9 +255,9 @@ extern "C" int nsb_train_fwd_bwd(const float* rays_o, const float* rays_d, const
     const uint32_t f = flags | NSB_TRAINING;
     // independent Philox streams per (step, purpose)
     const uint64_t s_jit = step * 8 + 0, s_u = step * 8 + 1, s_nc = step * 8 + 2, s_nf = step * 8 + 3;
-    if (grads_f == grads_c + NSB_N_PARAMS) {          // one flat buffer (the trainer's layout): one memset
+    if (grads_c && grads_f == grads_c + NSB_N_PARAMS) {     // one flat buffer (the trainer's layout): one memset
         if (cudaMemsetAsync(grads_c, 0, 2 * sizeof(float) * NSB_N_PARAMS, st) != cudaSuccess) return NSB_E_CUDA;
-    } else {
+    } else if (grads_c) {
         if (cudaMemsetAsync(grads_c, 0, sizeof(float) * NSB_N_PARAMS, st) != cudaSuccess) return NSB_E_CUDA;
         if (cudaMemsetAsync(grads_f, 0, sizeof(float) * NSB_N_PARAMS, st) != cudaSuccess) return NSB_E_CUDA;
     }
@@ -289,15 +314,41 @@ extern "C" int nsb_train_fwd_bwd(const float* rays_o, const float* rays_d, const
     // leave idle in their last round.  The loss scalars are computed at the head of the side stream.  Fork/join through events,
     // so the sequence stays graph-capturable.
     if (side && !fork()) return NSB_E_CUDA;
+    // With ray gradients each pass's field backward also writes its encoding gradients, which nsb_encode_bwd_rays reduces to the
+    // rays: the fine pass's straight into the outputs, the coarse pass's (side stream) into a buffer added after the join.
     NSB_TRY(composite_bwd(true, stream));
-    NSB_TRY(nsb_field_bwd(t.d_raw, packed_f, grads_f, t.field_f, t.field_f_bytes, Qf, mode, stream));
+    NSB_TRY(nsb_field_bwd_ex(t.d_raw, packed_f, grads_f, t.d_ep_f, t.d_ed_f, t.field_f, t.field_f_bytes, Qf, mode, stream));
+    if (ray_grads)
+        NSB_TRY(nsb_encode_bwd_rays(t.d_ep_f, t.d_ed_f, rays_o, rays_d, t.z_all, ray_norm, viewdirs, d_rays_o, d_rays_d, d_viewdirs,
+                                    B, Nt, stream));
     NSB_TRY(nsb_mse_loss(t.comp_c, t.comp_f, target, nullptr, nullptr, scalars, B, grad_scale, sstream));
     NSB_TRY(composite_bwd(false, sstream));
-    NSB_TRY(nsb_field_bwd(t.d_raw_c, packed_c, grads_c, t.field_c, t.field_c_bytes, Qc, mode, sstream));
+    NSB_TRY(nsb_field_bwd_ex(t.d_raw_c, packed_c, grads_c, t.d_ep_c, t.d_ed_c, t.field_c, t.field_c_bytes, Qc, mode, sstream));
+    float* dr_c = t.d_rays_c;
+    if (ray_grads)
+        NSB_TRY(nsb_encode_bwd_rays(t.d_ep_c, t.d_ed_c, rays_o, rays_d, t.zc, ray_norm, viewdirs, d_rays_o ? dr_c : nullptr,
+                                    d_rays_d ? dr_c + 3 * B : nullptr, d_viewdirs ? dr_c + 6 * B : nullptr, B, Nc, sstream));
     if (side && !join()) return NSB_E_CUDA;
+    if (ray_grads) {
+        const int64_t want = cdiv(3 * B, 256), cap = (int64_t)num_sms() * 8;
+        add_coarse_ray_grads_kernel<<<(int)(want < cap ? want : cap), 256, 0, st>>>(d_rays_o, d_rays_d, d_viewdirs, dr_c, 3 * B);
+        NSB_LAUNCH_CHECK("add_coarse_ray_grads_kernel");
+    }
     if (comp_c && cudaMemcpyAsync(comp_c, t.comp_c, B * 12, cudaMemcpyDeviceToDevice, st) != cudaSuccess) return NSB_E_CUDA;
     if (comp_f && cudaMemcpyAsync(comp_f, t.comp_f, B * 12, cudaMemcpyDeviceToDevice, st) != cudaSuccess) return NSB_E_CUDA;
     return NSB_OK;
+}
+
+extern "C" int nsb_train_fwd_bwd(const float* rays_o, const float* rays_d, const float* ray_norm, const float* viewdirs,
+                                 const float* target, const void* packed_c, const void* packed_f, float* grads_c,
+                                 float* grads_f, float* scalars, float* comp_c, float* comp_f, void* ws, size_t ws_bytes,
+                                 int64_t B, int Nc, int Nf, float near_, float far_, float noise_std, uint32_t flags,
+                                 int det_fine, int mode, float grad_scale, uint64_t seed, uint64_t step, const float* U,
+                                 const float* u_fine, const float* noise_c, const float* noise_f, void* stream) {
+    if (!grads_c || !grads_f) return NSB_E_BADARG;
+    return nsb_train_fwd_bwd_ex(rays_o, rays_d, ray_norm, viewdirs, target, packed_c, packed_f, grads_c, grads_f, scalars, comp_c, comp_f,
+                                ws, ws_bytes, B, Nc, Nf, near_, far_, noise_std, flags, det_fine, mode, grad_scale, seed, step, U, u_fine,
+                                noise_c, noise_f, nullptr, nullptr, nullptr, stream);
 }
 
 // ---------------------------------------------------------------------------------------------------

@@ -105,6 +105,163 @@ __global__ void sample_pixel_batch_kernel(const float* __restrict__ images, int 
     }
 }
 
+// ---- camera-ray backward: d(six outputs) -> d c2w[:3,:4] per frame (pose refinement, iNeRF / BARF) ----
+// Per ray, the forward of ray_from_pixel is recomputed in registers with the same expressions (this file is compiled with
+// -fmad=false, so the recomputed intermediates are bitwise the forward's), then differentiated by hand:
+//   d = R dc,  nrm = |d|,  du = d / (nrm + 1e-9)                                   (world outputs; o_world = t)
+//   NDC: tn = -(near + t_z) / (d_z + 1e-9), ow = t + tn d, oz = ow_z + 1e-9, dz = d_z + 1e-9, om / D as the forward,
+//        nn = |D|, dm = D / max(nn, 1e-12)                                          (F.normalize's backward)
+// and dL/dR[r][k] = dL/dd_r * dc_k, dL/dt_r.  Rays are summed into their frame's 12-vector without atomics: each block owns
+// one [F,12] slice of block partials in the workspace and adds its tiles of 256 rays to it in tile order (one warp per
+// (frame, component) pair, a fixed butterfly over the tile); camera_rays_bwd_reduce_kernel then sums the block partials in
+// block order.  The result is bitwise repeatable, and a frame no ray belongs to gets exactly zero.
+struct RayGrad { const float *ow, *du, *nrm, *om, *dm, *nm; };
+
+constexpr int kRaysBwdThreads = 256;
+constexpr int kRaysBwdMaxBlocks = 296;
+static inline int rays_bwd_blocks(int64_t n) { return (int)(cdiv(n, kRaysBwdThreads) < kRaysBwdMaxBlocks ? cdiv(n, kRaysBwdThreads) : kRaysBwdMaxBlocks); }
+
+__device__ __forceinline__ float opt_ld(const float* p, int64_t i) { return p ? p[i] : 0.0f; }
+
+__device__ __forceinline__ void ray_bwd_from_pixel(const RayCam& c, float x, float y, int H, int W, int pixel_center, int as_ndc,
+                                                   float near_plane, const RayGrad& g, int64_t i, float out[12]) {
+    if (pixel_center) { x += 0.5f; y += 0.5f; }
+    const float xc = (x - c.cx) / c.fx, yc = (y - c.cy) / c.fy;
+    const float dc[3] = {xc, c.sy_cam * yc, c.sz_cam};
+    float d[3];
+#pragma unroll
+    for (int r = 0; r < 3; ++r) d[r] = dc[0] * c.R[3 * r] + dc[1] * c.R[3 * r + 1] + dc[2] * c.R[3 * r + 2];
+    const float nrm = sqrtf(d[0] * d[0] + d[1] * d[1] + d[2] * d[2]);
+    const float inv = nrm + 1e-9f;
+    float gd[3] = {0.f, 0.f, 0.f}, gt[3], gdu[3];
+#pragma unroll
+    for (int r = 0; r < 3; ++r) { gt[r] = opt_ld(g.ow, 3 * i + r); gdu[r] = opt_ld(g.du, 3 * i + r); }
+    float gnrm = opt_ld(g.nrm, i);
+    if (!as_ndc) {                                             // marching rays are the world rays
+#pragma unroll
+        for (int r = 0; r < 3; ++r) { gt[r] += opt_ld(g.om, 3 * i + r); gdu[r] += opt_ld(g.dm, 3 * i + r); }
+        gnrm += opt_ld(g.nm, i);
+    } else {
+        const float sx = 2.0f * c.fx / (float)W, sy = 2.0f * c.fx / (float)H;
+        const float e = d[2] + 1e-9f;
+        const float tn = -(near_plane + c.t[2]) / e;
+        const float ow[3] = {c.t[0] + tn * d[0], c.t[1] + tn * d[1], c.t[2] + tn * d[2]};
+        const float oz = ow[2] + 1e-9f, dz = e;
+        const float D[3] = {-sx * (d[0] / dz - ow[0] / oz), -sy * (d[1] / dz - ow[1] / oz), -2.0f * near_plane / oz};
+        const float nn = sqrtf(D[0] * D[0] + D[1] * D[1] + D[2] * D[2]);
+        const float dn = fmaxf(nn, 1e-12f);
+        const float gdm[3] = {opt_ld(g.dm, 3 * i), opt_ld(g.dm, 3 * i + 1), opt_ld(g.dm, 3 * i + 2)};
+        const float gom[3] = {opt_ld(g.om, 3 * i), opt_ld(g.om, 3 * i + 1), opt_ld(g.om, 3 * i + 2)};
+        // dm = D / max(nn, eps), nm = nn
+        const float gD_dot = gdm[0] * D[0] + gdm[1] * D[1] + gdm[2] * D[2];
+        const float kD = nn > 0.f ? (opt_ld(g.nm, i) - (nn > 1e-12f ? gD_dot / (dn * dn) : 0.f)) / nn : 0.f;
+        float gD[3];
+#pragma unroll
+        for (int r = 0; r < 3; ++r) gD[r] = gdm[r] / dn + D[r] * kD;
+        const float s[2] = {sx, sy};
+        const float oz2 = oz * oz;
+        float gow[3] = {0.f, 0.f, 0.f}, goz = 0.f, gdz = 0.f;
+#pragma unroll
+        for (int r = 0; r < 2; ++r) {
+            // D_r = -s (d_r / dz - ow_r / oz),  om_r = -s ow_r / oz
+            gd[r] += -s[r] * gD[r] / dz;
+            gdz += s[r] * gD[r] * d[r] / (dz * dz);
+            gow[r] += s[r] * (gD[r] - gom[r]) / oz;
+            goz += s[r] * (gom[r] - gD[r]) * ow[r] / oz2;
+        }
+        goz += 2.0f * near_plane * (gD[2] - gom[2]) / oz2;     // D_2 = -2 near / oz,  om_2 = 1 + 2 near / oz
+        gow[2] += goz;
+        gd[2] += gdz;
+        // ow = t + tn d,  tn = -(near + t_z) / e
+        const float gtn = gow[0] * d[0] + gow[1] * d[1] + gow[2] * d[2];
+#pragma unroll
+        for (int r = 0; r < 3; ++r) { gt[r] += gow[r]; gd[r] += tn * gow[r]; }
+        gt[2] += -gtn / e;
+        gd[2] += gtn * (near_plane + c.t[2]) / (e * e);
+    }
+    // du = d / (nrm + 1e-9),  nrm = |d|
+    const float gdu_d = gdu[0] * d[0] + gdu[1] * d[1] + gdu[2] * d[2];
+    gnrm += -gdu_d / (inv * inv);
+    const float kn = nrm > 0.f ? gnrm / nrm : 0.f;
+#pragma unroll
+    for (int r = 0; r < 3; ++r) gd[r] += gdu[r] / inv + d[r] * kn;
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+#pragma unroll
+        for (int k = 0; k < 3; ++k) out[4 * r + k] = gd[r] * dc[k];
+        out[4 * r + 3] = gt[r];
+    }
+}
+
+__global__ void __launch_bounds__(kRaysBwdThreads)
+camera_rays_bwd_kernel(int H, int W, const float* __restrict__ Ks, const float* __restrict__ c2ws, int F, const int* __restrict__ fids,
+                       float sy_cam, float sz_cam, int pixel_center, int as_ndc, float near_plane, const float* __restrict__ pixels_xy,
+                       int64_t n, RayGrad g, float* __restrict__ partial) {
+    __shared__ float vals[12][kRaysBwdThreads];
+    __shared__ int tile_fid[kRaysBwdThreads];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = kRaysBwdThreads / 32;
+    const int pairs = 12 * F;
+    float* mine = partial + (int64_t)blockIdx.x * pairs;
+    if (lane == 0)
+        for (int p = warp; p < pairs; p += nwarps) mine[p] = 0.f;
+    const int64_t tiles = (n + kRaysBwdThreads - 1) / kRaysBwdThreads;
+    for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
+        const int64_t i = tile * kRaysBwdThreads + tid;
+        int f = -1;
+        float out[12];
+        if (i < n) {
+            f = fids ? fids[i] : 0;
+            if (f < 0 || f >= F) f = -1;                       // a ray of no frame contributes nothing
+        }
+        if (f >= 0) {
+            float x, y;
+            if (pixels_xy) { x = pixels_xy[2 * i]; y = pixels_xy[2 * i + 1]; }
+            else { x = (float)(i % W); y = (float)(i / W); }
+            RayCam c;
+            c.fx = Ks[4 * f]; c.fy = Ks[4 * f + 1]; c.cx = Ks[4 * f + 2]; c.cy = Ks[4 * f + 3];
+#pragma unroll
+            for (int r = 0; r < 3; ++r) {
+#pragma unroll
+                for (int k = 0; k < 3; ++k) c.R[3 * r + k] = c2ws[12 * f + 4 * r + k];
+                c.t[r] = c2ws[12 * f + 4 * r + 3];
+            }
+            c.sy_cam = sy_cam; c.sz_cam = sz_cam;
+            ray_bwd_from_pixel(c, x, y, H, W, pixel_center, as_ndc, near_plane, g, i, out);
+        } else {
+#pragma unroll
+            for (int k = 0; k < 12; ++k) out[k] = 0.f;
+        }
+#pragma unroll
+        for (int k = 0; k < 12; ++k) vals[k][tid] = out[k];
+        tile_fid[tid] = f;
+        __syncthreads();
+        for (int p = warp; p < pairs; p += nwarps) {
+            const int pf = p / 12, pc = p - 12 * pf;
+            float s = 0.f;
+            bool hit = false;
+#pragma unroll
+            for (int k = lane; k < kRaysBwdThreads; k += 32)
+                if (tile_fid[k] == pf) { s += vals[pc][k]; hit = true; }
+            if (__any_sync(0xffffffffu, hit)) {
+                s = warp_sum(s);
+                if (lane == 0) mine[p] += s;
+            }
+        }
+        __syncthreads();
+    }
+}
+
+// d_c2ws[p] = sum over blocks of partial[block][p], block order; one warp per (frame, component)
+__global__ void camera_rays_bwd_reduce_kernel(const float* __restrict__ partial, int blocks, int pairs, float* __restrict__ d_c2ws) {
+    const int lane = threadIdx.x & 31;
+    const int p = (int)((blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5);
+    if (p >= pairs) return;
+    float s = 0.f;
+    for (int b = lane; b < blocks; b += 32) s += partial[(int64_t)b * pairs + p];
+    s = warp_sum(s);
+    if (lane == 0) d_c2ws[p] = s;
+}
+
 // ---- eval output path (SURVEY 8f rank 4): what validation_renderer.py:485-533 + render_utils.py:28-47 do with a frame ----
 // u8 = (clamp(x, 0, 1) * 255 + 0.5) truncated  (two roundings: this file is compiled with -fmad=false, like numpy)
 __device__ __forceinline__ uint8_t to_u8(float x) { return (uint8_t)(fminf(fmaxf(x, 0.0f), 1.0f) * 255.0f + 0.5f); }
@@ -186,6 +343,36 @@ extern "C" int nsb_camera_rays(int H, int W, const float* K_host, const float* c
     camera_rays_kernel<<<(int)(want < cap ? want : cap), 256, 0, as_stream(stream)>>>(
         c, H, W, pixels_xy, n, pixel_center, as_ndc, near_plane, o_world, d_world_unit, d_world_norm, o_march, d_march_unit, d_march_norm);
     NSB_LAUNCH_CHECK("camera_rays_kernel");
+    return NSB_OK;
+}
+
+extern "C" size_t nsb_camera_rays_bwd_workspace_bytes(int64_t n, int F) {
+    if (n <= 0 || F < 1) return 0;
+    return align_up((size_t)rays_bwd_blocks(n) * 12 * (size_t)F * sizeof(float), 256);
+}
+
+extern "C" int nsb_camera_rays_bwd(int H, int W, const float* Ks, const float* c2ws, int F, const int* fids, int convention,
+                                   int pixel_center, int as_ndc, float near_plane, const float* pixels_xy, int64_t n,
+                                   const float* g_o_world, const float* g_d_world_unit, const float* g_d_world_norm,
+                                   const float* g_o_march, const float* g_d_march_unit, const float* g_d_march_norm,
+                                   float* d_c2ws, void* ws, size_t ws_bytes, void* stream) {
+    if (!Ks || !c2ws || !d_c2ws || F < 1 || H < 1 || W < 1 || n < 0 || convention < 0 || convention > 2) return NSB_E_BADARG;
+    if (!g_o_world && !g_d_world_unit && !g_d_world_norm && !g_o_march && !g_d_march_unit && !g_d_march_norm) return NSB_E_BADARG;
+    if (!pixels_xy && n != (int64_t)H * W) return NSB_E_BADARG;
+    cudaStream_t st = as_stream(stream);
+    if (n == 0)
+        return cudaMemsetAsync(d_c2ws, 0, (size_t)F * 12 * sizeof(float), st) == cudaSuccess ? NSB_OK : NSB_E_CUDA;
+    if (!ws) return NSB_E_BADARG;
+    if (ws_bytes < nsb_camera_rays_bwd_workspace_bytes(n, F)) return NSB_E_WORKSPACE;
+    const int blocks = rays_bwd_blocks(n), pairs = 12 * F;
+    float* partial = static_cast<float*>(ws);
+    const RayGrad g{g_o_world, g_d_world_unit, g_d_world_norm, g_o_march, g_d_march_unit, g_d_march_norm};
+    camera_rays_bwd_kernel<<<blocks, kRaysBwdThreads, 0, st>>>(H, W, Ks, c2ws, F, fids, convention == 1 ? 1.0f : -1.0f,
+                                                               convention == 0 ? -1.0f : 1.0f, pixel_center, as_ndc, near_plane,
+                                                               pixels_xy, n, g, partial);
+    NSB_LAUNCH_CHECK("camera_rays_bwd_kernel");
+    camera_rays_bwd_reduce_kernel<<<(int)cdiv((int64_t)pairs * 32, 256), 256, 0, st>>>(partial, blocks, pairs, d_c2ws);
+    NSB_LAUNCH_CHECK("camera_rays_bwd_reduce_kernel");
     return NSB_OK;
 }
 

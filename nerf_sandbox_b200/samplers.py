@@ -11,7 +11,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .rays import _CONV
+from .rays import _CONV, PoseRaysFn
 
 
 class RandomPixelRaySampler:
@@ -57,19 +57,44 @@ class RandomPixelRaySampler:
             return int(H * 0.5 * (1.0 - f)), int(H * 0.5 * (1.0 + f)), int(W * 0.5 * (1.0 - f)), int(W * 0.5 * (1.0 + f))
         return 0, H, 0, W
 
-    def next_batch(self, with_pixels: bool = False) -> Dict[str, torch.Tensor]:
+    def next_batch(self, with_pixels: bool = False, c2ws: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+        """One batch of `rays_per_batch` rays.  ``c2ws`` ([F,3,4] or [F,4,4] CUDA tensor on the sampler's device) replaces the
+        scene's poses for this draw; when it requires grad (and grad mode is on) the six ray outputs backpropagate into it
+        through nsb_camera_rays_bwd, using the pixels and frame ids this draw made -- per-frame pose refinement (BARF-style).
+        The gradient is exact for the rays themselves.  Downstream, the render path gives no gradient to the ray norms, so for
+        NDC rays (``as_ndc``), whose marching norm depends on the pose, the pose gradient of a rendering loss is incomplete."""
+        poses = self._c2ws
+        if c2ws is not None:
+            dev = self.device if self.device.index is not None else torch.device("cuda", torch.cuda.current_device())
+            if not isinstance(c2ws, torch.Tensor) or c2ws.device != dev:
+                raise ValueError(f"c2ws must be a tensor on {self.device}")
+            if c2ws.dim() != 3 or c2ws.shape[0] != self.F or tuple(c2ws.shape[1:]) not in {(3, 4), (4, 4)}:
+                raise ValueError(f"c2ws must be [{self.F},3,4] or [{self.F},4,4], got {tuple(c2ws.shape)}")
+            poses = c2ws.detach()[:, :3, :4].to(torch.float32).contiguous().reshape(self.F, 12)
+        grad = c2ws is not None and torch.is_grad_enabled() and c2ws.requires_grad
         h0, h1, w0, w1 = self._current_crop_bounds()
         fid = int(self._rng.integers(self.F)) if self.sample_from_single_frame else -1
         B, dev = self.B, self.device
         e = lambda k: torch.empty((B, k), device=dev, dtype=torch.float32)
-        rgb, ow, du, dn, om, dm, mn = e(3), e(3), e(3), e(1), e(3), e(3), e(1)
-        px = e(2) if with_pixels else None
-        fids = torch.empty((B,), device=dev, dtype=torch.int32) if with_pixels else None
-        _lib.check(_lib.lib().nsb_sample_pixel_batch(
-            _lib.ptr(self._imgs), self.F, self.H, self.W, self.C, _lib.ptr(self._Ks), _lib.ptr(self._c2ws), fid, h0, h1, w0, w1,
-            int(self.white_bkgd), _CONV[self.convention], int(self.as_ndc), self.near_plane, B, self.seed, self._global_step,
-            _lib.ptr(rgb), _lib.ptr(px), _lib.ptr(fids), _lib.ptr(ow), _lib.ptr(du), _lib.ptr(dn), _lib.ptr(om), _lib.ptr(dm),
-            _lib.ptr(mn), torch.cuda.current_stream(dev).cuda_stream), "nsb_sample_pixel_batch")
+        rgb = e(3)
+        px = e(2) if (with_pixels or grad) else None                 # the backward needs what this draw picked
+        fids = torch.empty((B,), device=dev, dtype=torch.int32) if (with_pixels or grad) else None
+
+        def run():
+            rays = (e(3), e(3), e(1), e(3), e(3), e(1))
+            _lib.check(_lib.lib().nsb_sample_pixel_batch(
+                _lib.ptr(self._imgs), self.F, self.H, self.W, self.C, _lib.ptr(self._Ks), _lib.ptr(poses), fid, h0, h1, w0, w1,
+                int(self.white_bkgd), _CONV[self.convention], int(self.as_ndc), self.near_plane, B, self.seed, self._global_step,
+                _lib.ptr(rgb), _lib.ptr(px), _lib.ptr(fids), *[_lib.ptr(t) for t in rays],
+                torch.cuda.current_stream(dev).cuda_stream), "nsb_sample_pixel_batch")
+            return rays
+
+        if grad:
+            ow, du, dn, om, dm, mn = PoseRaysFn.apply(c2ws, run, dict(
+                H=self.H, W=self.W, Ks=self._Ks, c2ws=poses, convention=self.convention, pixel_center=True, as_ndc=self.as_ndc,
+                near_plane=self.near_plane, pixels_xy=px, fids=fids))
+        else:
+            ow, du, dn, om, dm, mn = run()
         self._global_step += 1
         batch = {"rgb": rgb, "rays_o_world": ow, "rays_d_world_unit": du, "rays_d_world_norm": dn, "rays_o_marching": om,
                  "rays_d_marching_unit": dm, "rays_d_marching_norm": mn}                     # samplers.py:193-201

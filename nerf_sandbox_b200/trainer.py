@@ -28,15 +28,26 @@ def mse2psnr(mse: torch.Tensor) -> torch.Tensor:                       # trainer
 
 
 class _FusedStepFn(torch.autograd.Function):
-    """loss = mse(comp_c)+mse(comp_f); forward already ran the backward kernels, so ``backward`` only scales."""
+    """loss = mse(comp_c)+mse(comp_f); forward already ran the backward kernels, so ``backward`` only scales.  The ray tensors
+    (rays_o_marching, rays_d_marching_unit, rays_d_world_unit) are explicit inputs: when one requires grad the step also
+    computes the loss's gradient w.r.t. them (nsb_train_fwd_bwd_ex)."""
 
     @staticmethod
-    def forward(ctx, tr, batch, draws, *params):
+    def forward(ctx, tr, batch, draws, grad_mode, rays_o, rays_d, viewdirs, *params):
         # gradients go to a buffer of this call's own (never the trainer's shared / peer-visible buffers): a later
         # _train_step(), step() or step_graph() before loss.backward() cannot change what backward() returns
+        want = [grad_mode and t.requires_grad for t in (rays_o, rays_d, viewdirs)]
+        ray_grads = None
         grads = torch.empty(2 * _lib.N_PARAMS, device=tr.device, dtype=torch.float32)
-        scal, comp_c, comp_f = tr._fwd_bwd(batch, draws, grad_scale=1.0, grads=grads)
+        if any(want):
+            ray_grads = tuple(torch.empty((t.shape[0], 3), device=tr.device, dtype=torch.float32) if w else None
+                              for t, w in zip((rays_o, rays_d, viewdirs), want))
+            if not any(p.requires_grad for p in params):
+                grads = None                                     # frozen field: no weight-gradient kernel runs
+        scal, comp_c, comp_f = tr._fwd_bwd(batch, draws, grad_scale=1.0, grads=grads, ray_grads=ray_grads)
         ctx.tr = tr
+        ctx.ray_grads = ray_grads
+        ctx.ray_meta = [(t.shape, t.dtype) for t in (rays_o, rays_d, viewdirs)]
         ctx.save_for_backward(grads)
         ctx.mark_non_differentiable(comp_c, comp_f)
         return scal[0].clone(), scal[1].clone(), comp_c, comp_f
@@ -46,9 +57,13 @@ class _FusedStepFn(torch.autograd.Function):
         tr = ctx.tr
         (grads,) = ctx.saved_tensors
         n = _lib.N_PARAMS
-        gc = tr.nerf_c.unflatten(grads[:n] * g_loss)
-        gf = tr.nerf_f.unflatten(grads[n:] * g_loss)
-        return (None, None, None) + tuple(gc) + tuple(gf)
+        if grads is None:
+            pg = (None,) * (len(ctx.needs_input_grad) - 7)
+        else:
+            pg = tuple(tr.nerf_c.unflatten(grads[:n] * g_loss)) + tuple(tr.nerf_f.unflatten(grads[n:] * g_loss))
+        rg = (None, None, None) if ctx.ray_grads is None else tuple(
+            None if g is None else (g * g_loss).reshape(m[0]).to(m[1]) for g, m in zip(ctx.ray_grads, ctx.ray_meta))
+        return (None, None, None, None) + rg + pg
 
 
 class VanillaTrainer:
@@ -160,40 +175,54 @@ class VanillaTrainer:
         return ((_lib.WHITE_BKGD if self.white_bkgd else 0) | (_lib.INFINITE_LAST_BIN if self.infinite_last_bin else 0)
                 | (_lib.SIGMA_SOFTPLUS if self.sigma_activation == "softplus" else 0))
 
-    def _workspace(self, B):
-        need = _lib.lib().nsb_train_workspace_bytes(B, self.nc, self.nf, self.mode)
+    def _workspace(self, B, ray_grads=False):
+        need = _lib.lib().nsb_train_workspace_bytes_ex(B, self.nc, self.nf, self.mode, int(ray_grads))
         if self._ws is None or self._ws.numel() < need:
             self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
             self._graphs = None                    # captured graphs hold the old workspace address: recapture on next use
         return self._ws, need
 
-    def _fwd_bwd(self, batch, draws=None, grad_scale=1.0, grads=None):
+    def _fwd_bwd(self, batch, draws=None, grad_scale=1.0, grads=None, ray_grads=None):
         """nsb_train_fwd_bwd: fills `grads` (default: this step's self.grads_c/grads_f) and self.scalars; returns
-        (scalars, comp_c, comp_f)."""
+        (scalars, comp_c, comp_f).  ray_grads = (d_rays_o, d_rays_d, d_viewdirs) [B,3] fp32 outputs, each optional: then
+        nsb_train_fwd_bwd_ex, and `grads` may be None (a frozen field)."""
         L = _lib.lib()
         o, d, rn, vd, tgt = (_lib.f32c(batch[k]) for k in BATCH_KEYS)
         B = o.shape[0]
-        ws, wsb = self._workspace(B)
+        ws, wsb = self._workspace(B, ray_grads is not None)
         comp_c = torch.empty((B, 3), device=self.device); comp_f = torch.empty((B, 3), device=self.device)
         draws = draws or {}
         g = lambda k: None if draws.get(k) is None else _lib.f32c(draws[k])
         n = _lib.N_PARAMS
-        grads_c, grads_f = (self.grads_c, self.grads_f) if grads is None else (grads[:n], grads[n:])
-        _lib.check(L.nsb_train_fwd_bwd(
-            _lib.ptr(o), _lib.ptr(d), _lib.ptr(rn.reshape(B)), _lib.ptr(vd), _lib.ptr(tgt),
-            _lib.ptr(self.nerf_c.packed(for_inference=False)), _lib.ptr(self.nerf_f.packed(for_inference=False)), _lib.ptr(grads_c), _lib.ptr(grads_f),
-            _lib.ptr(self.scalars), _lib.ptr(comp_c), _lib.ptr(comp_f), _lib.ptr(ws), wsb, B, self.nc, self.nf,
-            self.samp_near, self.samp_far, self.raw_noise_std, self._flags(), int(self.det_fine), self.mode,
-            float(grad_scale), self.seed, self.global_step, _lib.ptr(g("U")), _lib.ptr(g("u_fine")),
-            _lib.ptr(g("noise_c")), _lib.ptr(g("noise_f")), _lib.stream()), "nsb_train_fwd_bwd")
+        if ray_grads is not None:
+            grads_c, grads_f = (None, None) if grads is None else (grads[:n], grads[n:])
+        else:
+            grads_c, grads_f = (self.grads_c, self.grads_f) if grads is None else (grads[:n], grads[n:])
+        args = (_lib.ptr(o), _lib.ptr(d), _lib.ptr(rn.reshape(B)), _lib.ptr(vd), _lib.ptr(tgt),
+                _lib.ptr(self.nerf_c.packed(for_inference=False)), _lib.ptr(self.nerf_f.packed(for_inference=False)), _lib.ptr(grads_c),
+                _lib.ptr(grads_f), _lib.ptr(self.scalars), _lib.ptr(comp_c), _lib.ptr(comp_f), _lib.ptr(ws), wsb, B, self.nc, self.nf,
+                self.samp_near, self.samp_far, self.raw_noise_std, self._flags(), int(self.det_fine), self.mode,
+                float(grad_scale), self.seed, self.global_step, _lib.ptr(g("U")), _lib.ptr(g("u_fine")),
+                _lib.ptr(g("noise_c")), _lib.ptr(g("noise_f")))
+        if ray_grads is None:
+            _lib.check(L.nsb_train_fwd_bwd(*args, _lib.stream()), "nsb_train_fwd_bwd")
+        else:
+            _lib.check(L.nsb_train_fwd_bwd_ex(*args, *[_lib.ptr(t) for t in ray_grads], _lib.stream()), "nsb_train_fwd_bwd_ex")
         return self.scalars, comp_c, comp_f
 
     # ---- reference-compatible step ---------------------------------------------------------------------
     def _train_step(self, batch, draws=None) -> dict:
         """Same contract as Trainer._train_step (trainer.py:876-1013): ``loss`` carries autograd history to the
-        48 parameters, so ``loss.backward(); torch.optim.Adam(...).step()`` works unchanged."""
-        loss, psnr, comp_c, comp_f = _FusedStepFn.apply(self, batch, draws, *self.nerf_c.ordered_params(),
-                                                        *self.nerf_f.ordered_params())
+        48 parameters, so ``loss.backward(); torch.optim.Adam(...).step()`` works unchanged.
+
+        When ``rays_o_marching``, ``rays_d_marching_unit`` or ``rays_d_world_unit`` requires grad (and grad mode is on), the
+        loss also backpropagates into them -- e.g. to poses through ``RandomPixelRaySampler.next_batch(c2ws=...)`` or
+        ``get_camera_rays``.  The ray norms and z samples get no gradient.  For world-space rays that loses nothing under a
+        rigid pose update (|R d_cam| does not depend on R); for NDC rays the marching norm depends on the pose, so their pose
+        gradient is incomplete.  When no NeRF parameter requires grad, only the ray gradients are computed."""
+        loss, psnr, comp_c, comp_f = _FusedStepFn.apply(self, batch, draws, torch.is_grad_enabled(), batch["rays_o_marching"],
+                                                        batch["rays_d_marching_unit"], batch["rays_d_world_unit"],
+                                                        *self.nerf_c.ordered_params(), *self.nerf_f.ordered_params())
         return {"loss": loss, "psnr": psnr.detach(), "comp_f": comp_f.detach(), "comp_c": comp_c.detach()}
 
     # ---- fast path ---------------------------------------------------------------------------------------
